@@ -2,6 +2,7 @@
 """bench.py -- SVI throughput of the `bean run` hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--scaling strong|weak] [--workload c5_genome_scale] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one complete SVI step (guide sampling + ELBO forward/backward + ClippedAdam) of the MixtureNormal sorting
 model over one synthetic screen.  Workload: the configuration BASELINE.json's target is quoted on, c5 = 1M guides x 8
@@ -12,6 +13,11 @@ screen is split into contiguous variant blocks (`dist.shard_variants`), every ra
 ELBO scalars -- the only quantity of this model that crosses ranks (SURVEY section 8e) -- are all-reduced over NCCL in
 batches of <= 100 steps INSIDE the timed region (the reference prints the loss every 100 steps, run.py:378).
 `--scaling weak` gives every rank its own 1M-guide screen instead.
+
+`--dump-outputs DIR` (one GPU) writes what the timed steps hand a caller, taken right after the last timed step: the ELBO
+loss of every timed step (`DIR/loss.npy`, float64) and the fitted parameters under the reference's names
+(`DIR/<name>.npy`, in the engine's dtype).  The screen and the engine's draws are seeded, so two builds run with the
+same arguments can be compared array for array.
 
 Prints ONE JSON line (rank 0).  `--impl reference` times the CPU oracle port of the reference path on the box's host
 cores at the FULL workload size (pyro is not installable here, so the reference itself cannot run; SURVEY 8c).
@@ -43,6 +49,7 @@ SURVIVAL = ("c4_survival", "c4_survival_small")
 BASELINE_MD_PUBLISHED = None  # BASELINE.md holds no published number for this metric -> vs_baseline null
 LOSS_BATCH = 100              # steps per ELBO all-reduce (reference print cadence, bean/model/run.py:378)
 GUIDE_PROFILE = os.path.join(ROOT, "profiles", "r2_guide_metrics.txt")  # ncu --set full capture of the dominant kernel
+DUMP_LIMIT = 64 << 20         # bytes --dump-outputs may write in all
 
 
 def algorithmic_bytes_per_guide(R, B, L, guides_per_variant, itemsize=4):
@@ -153,9 +160,22 @@ def make_bench_engine(workload, data, dev, dtype, num_steps, seed, off):
                      variant_offset=off["variant_offset"])
 
 
+def dump_outputs(path, arrays):
+    """Writes every array as `path/<name>.npy`; refuses to write more than DUMP_LIMIT bytes in all."""
+    import numpy as np
+
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def oracle_step_time(data, steps, warmup=1, anomaly=True, max_seconds=240.0):
     """Seconds per SVI step of the CPU oracle (plain-torch restatement of the reference's MixtureNormal program); stops early
-    (after at least one timed step) once `max_seconds` have gone by."""
+    (after at least one timed step) once `max_seconds` have gone by; `max_seconds=None` times exactly `steps` steps."""
     from oracle import bean_oracle as O
 
     elbo_fn = O.elbo_survival_mixture_normal if getattr(data, "is_survival", False) else O.elbo_mixture_normal
@@ -166,7 +186,7 @@ def oracle_step_time(data, steps, warmup=1, anomaly=True, max_seconds=240.0):
     began = time.perf_counter()
     try:
         for t in range(warmup + steps):
-            if times and time.perf_counter() - began > max_seconds:
+            if max_seconds is not None and times and time.perf_counter() - began > max_seconds:
                 break
             t0 = time.perf_counter()
             loss, _ = elbo_fn(data, ps)
@@ -184,26 +204,35 @@ def oracle_step_time(data, steps, warmup=1, anomaly=True, max_seconds=240.0):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 100; the reference arm by default stops at --cpu-max-steps steps or after 240 s)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c5_genome_scale", choices=sorted(WORKLOADS))
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"])
     ap.add_argument("--dtype", default="f32", choices=["f32", "f64"])
     ap.add_argument("--cpu-sample-guides", type=int, default=0, help="0 = the full workload (default)")
-    ap.add_argument("--cpu-max-steps", type=int, default=25, help="upper bound on the reference arm's timed steps")
+    ap.add_argument("--cpu-max-steps", type=int, default=25, help="upper bound on the reference arm's timed steps when --steps is not given")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--full-run-steps", type=int, default=4000, help="length of the complete run timed after the K steps (0 = skip)")
     ap.add_argument("--burn-in", type=int, default=300,
                     help="untimed SVI steps before the timed region: a step gets slower over the first ~300 steps of a run "
                          "(alpha_pi fits the low editing rates, more Dirichlet draws leave the saddle-point regime), so the "
                          "timed steps are taken where a real 2000-step run spends its time")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the losses of the timed steps and the parameters after the last one as DIR/<name>.npy")
     args = ap.parse_args()
+    steps_given = args.steps is not None
+    args.steps = args.steps if steps_given else 100
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     nv, gpv, nr = WORKLOADS[args.workload]
     survival = args.workload in SURVIVAL
     R, B, L = nr, (3 if survival else 4), 2
@@ -240,12 +269,14 @@ def main():
         data = build_data(args.workload, seed=101)
         if args.cpu_sample_guides and args.cpu_sample_guides < data.n_guides:
             data = data[torch.arange(args.cpu_sample_guides)]
-        steps = max(1, min(args.steps, args.cpu_max_steps))
-        sec = oracle_step_time(data, steps, warmup=max(min(args.warmup, 2), 1), anomaly=True)
+        # an explicit --steps is timed in full; by default the arm is capped, as one step of the full workload takes seconds
+        steps = args.steps if steps_given else max(1, min(args.steps, args.cpu_max_steps))
+        sec = oracle_step_time(data, steps, warmup=max(min(args.warmup, 2), 1), anomaly=True,
+                               max_seconds=None if steps_given else 240.0)
         sec_off = oracle_step_time(data, min(steps, 3), warmup=1, anomaly=False)
         cells = data.n_guides * R * B
         value = cells / sec
-        sample = (f"{'all' if data.n_guides == nv * gpv else 'first'} {data.n_guides} guides of the workload, <= {steps} timed SVI steps (240 s cap) of the "
+        sample = (f"{'all' if data.n_guides == nv * gpv else 'first'} {data.n_guides} guides of the workload, {steps if steps_given else f'<= {steps}'} timed SVI steps{'' if steps_given else ' (240 s cap)'} of the "
                   f"plain-torch oracle port on {torch.get_num_threads()} threads, torch anomaly mode ON as the reference leaves it "
                   f"(model.py:399): {sec * 1e3:.0f} ms/step; anomaly mode off: {sec_off * 1e3:.0f} ms/step; pyro itself is not "
                   "installable (no poutine overhead in this number)")
@@ -328,6 +359,9 @@ def main():
         ms_local = sum(a.elapsed_time(b) for a, b in evs)
     sampler.stop_flag = True
     sampler.join()
+    if args.dump_outputs:  # before the per-kernel timings below advance the engine further
+        outputs = {"loss": eng.loss[eng.step - args.steps:eng.step], **eng.params()}
+        dump_outputs(args.dump_outputs, {k: v.detach().cpu().numpy() for k, v in outputs.items()})
     ms = max_over_ranks(ms_local)
     steps_per_sec = args.steps / (ms * 1e-3)
     value = cells_per_step * steps_per_sec

@@ -2,7 +2,7 @@
 
 TEST INFRASTRUCTURE ONLY -- never imported by `crispr_bean_b200/` (the product).
 
-What it restates (all `file:line` relative to /root/reference):
+What it restates (all `file:line` relative to the original project's root):
   * `get_std_normal_prob`            bean/model/utils.py:34-76
   * `get_alpha`                      bean/model/utils.py:10-31
   * `scale_pi_by_accessibility`      bean/model/utils.py:79-178

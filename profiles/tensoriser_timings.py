@@ -4,7 +4,7 @@
 
 Mirror (crispr_bean_b200/data_class.py, vectorised, CSR tiling maps) beside the reference's own data classes
 (bean/preprocessing/data_class.py: per-guide Python loops, dense allele_to_edit), the latter executed in place
-through tests/refharness where /root/reference is mounted (build container only).  Equality of the two outputs is
+through tests/refharness where BEAN_REFERENCE_ROOT names a checkout of the original.  Equality of the two outputs is
 what tests/test_reference_golden.py checks; this script only reports wall-clock seconds on the host CPU.
 """
 import copy

@@ -1,4 +1,4 @@
-"""Regenerate tests/golden/* (run in the BUILD container, where /root/reference is mounted).
+"""Regenerate tests/golden/* (needs a checkout of the original project named by BEAN_REFERENCE_ROOT, tests/refharness).
 
 1. `var_mini.npz`: the only count fixture of the reference that is readable without anndata/h5py --
    tests/data/var_mini_{guides,samples,counts}.csv (30 guides x 2 replicates x 5 conditions) -- stored as
@@ -23,7 +23,9 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference/tests/data"
+from tests.refharness import REFERENCE_ROOT  # noqa: E402
+
+REF = os.path.join(REFERENCE_ROOT, "tests", "data")
 
 
 def main():

@@ -2,7 +2,7 @@
 
     python tests/golden/make_reference_golden.py          # writes tests/golden/ref_*.npz
 
-The reference's unmodified files are imported in place from /root/reference through tests/refharness
+The reference's unmodified files are imported in place from BEAN_REFERENCE_ROOT through tests/refharness
 (bean/preprocessing/data_class.py + get_alpha0.py + get_pi_alpha0.py for the tensors; bean/model/model.py,
 survival_model.py, utils.py, run.py for the programs).  pyro-ppl cannot be installed here, so the programs
 run on tests/refharness/pyro -- a restatement of the handful of pyro primitives they call (see its
@@ -24,7 +24,7 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 warnings.filterwarnings("ignore")
 
-from tests.refharness import load_reference  # noqa: E402
+from tests.refharness import REFERENCE_ROOT, load_reference  # noqa: E402
 from tests.refharness import golden as G  # noqa: E402
 
 
@@ -138,10 +138,10 @@ def tiling_cases(ns):
 def real_cases(ns):
     """The reference's own test screens (tests/data/*.h5ad, the inputs of its tests/test_run.py), read with the
     repo's HDF5 reader and prepared as cli/run.py does (guides sorted by target, negative controls from
-    `target_group`).  The screens travel inside the fixtures, so the tests never open /root/reference."""
+    `target_group`).  The screens travel inside the fixtures, so the tests never open the original project."""
     from crispr_bean_b200.screen import read_h5ad
 
-    ref_data = "/root/reference/tests/data/"
+    ref_data = os.path.join(REFERENCE_ROOT, "tests", "data") + os.sep
     m, sm, dc = ns.model, ns.survival_model, ns.data_class
 
     def load(name):

@@ -2,7 +2,7 @@
 
     python tests/golden/make_seam_fixture.py
 
-Runs the reference program (read in place from /root/reference, tests/refharness) with its count-likelihood block replaced by
+Runs the reference program (read in place from BEAN_REFERENCE_ROOT, tests/refharness) with its count-likelihood block replaced by
 `pyro.factor("guide_counts", count_ll(data, mu, sd, pi))` (INTEGRATION.md section A; tests/refharness/seam.py) on the screen of
 ref_mixture_small.npz with the same seed as that golden case, and records the seam's inputs (mu, sd (G, 2); pi (R, 1, G, 2)),
 the value the CPU oracle returns for them and its gradient w.r.t. the three inputs.  tests/test_integration_seam.py checks

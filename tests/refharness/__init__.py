@@ -1,6 +1,6 @@
-"""Loader that executes the reference's OWN source files (read in place from /root/reference, never copied)
-for golden-vector generation and cross-checks.  TEST INFRASTRUCTURE ONLY; available only where
-/root/reference exists (this container) -- the GPU box and the `-m gpu` tests use the committed vectors.
+"""Loader that executes the reference's OWN source files (read in place from a checkout of the original project named by
+the environment variable BEAN_REFERENCE_ROOT, never copied) for golden-vector generation and cross-checks.  TEST
+INFRASTRUCTURE ONLY; the tests that need it skip without that checkout, the rest of the suite uses the committed vectors.
 
 What is real and what is shimmed:
   real  (unmodified reference code): bean/model/{model,survival_model,utils,run,readwrite}.py,
@@ -15,12 +15,12 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("BEAN_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("BEAN_REFERENCE_ROOT", "")
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 def available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "bean", "model"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "bean", "model"))
 
 
 def load_reference():

@@ -4,7 +4,7 @@
 The reference source is read in place (never copied into the repo): the function's text is taken with `inspect`, everything
 from the first `with replicate_plate:` / `with bin_plate as b:` pair (bean/model/model.py:480-547: get_std_normal_prob ->
 mixture -> get_alpha x 2 -> DirichletMultinomial x 2) to the end of the function is cut, the two seam lines are appended, and the
-result is executed in the reference module's own namespace.  TEST INFRASTRUCTURE; needs /root/reference.
+result is executed in the reference module's own namespace.  TEST INFRASTRUCTURE; needs BEAN_REFERENCE_ROOT.
 """
 from __future__ import annotations
 

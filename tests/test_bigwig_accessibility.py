@@ -17,10 +17,10 @@ import torch
 
 from tests.support import bigwig
 from tests.support.accessibility import _get_accessibility_single, get_accessibility_guides
-from tests.refharness import available, load_reference
+from tests.refharness import REFERENCE_ROOT, available, load_reference
 
-REF_DATA = "/root/reference/tests/data"
-needs_data = pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference test data not mounted")
+REF_DATA = os.path.join(REFERENCE_ROOT, "tests", "data")
+needs_data = pytest.mark.skipif(not (REFERENCE_ROOT and os.path.isdir(REF_DATA)), reason="reference test data not mounted")
 
 
 def write_bigwig(path, chroms, sections, compress=True):

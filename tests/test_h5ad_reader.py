@@ -1,8 +1,8 @@
 """`read_h5ad` (crispr_bean_b200/screen.py) + the HDF5 subset reader (crispr_bean_b200/h5lite.py) on the reference's own
 `.h5ad` test screens (reference: bean/framework/ReporterScreen.py:read_h5ad, used by cli/run.py:62).
 
-The files are written by anndata/h5py and live under /root/reference/tests/data, which is mounted in the build
-container only: those tests skip elsewhere.  The screens they decode to are ALSO committed inside
+The files are written by anndata/h5py and live under tests/data of the original project (a checkout of it named by
+BEAN_REFERENCE_ROOT, tests/refharness): those tests skip without it.  The screens they decode to are ALSO committed inside
 tests/golden/ref_*real*.npz (with everything the reference computed from them), so the rest of the suite -- CPU and
 GPU -- exercises the decoded data without the files.
 """
@@ -15,10 +15,11 @@ import pytest
 from crispr_bean_b200 import h5lite
 from crispr_bean_b200.screen import MiniScreen, read_h5ad
 from tests.helpers import GOLDEN
+from tests.refharness import REFERENCE_ROOT
 from tests.refharness.golden import screen_from_arrays
 
-REF_DATA = "/root/reference/tests/data"
-needs_reference = pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference test data not mounted")
+REF_DATA = os.path.join(REFERENCE_ROOT, "tests", "data")
+needs_reference = pytest.mark.skipif(not (REFERENCE_ROOT and os.path.isdir(REF_DATA)), reason="reference test data not mounted")
 
 SHAPES = {  # file -> (guides, samples, rows of uns['allele_counts'])
     "var_mini_screen": (30, 10, 4926),

@@ -1,6 +1,6 @@
 """Program options the golden fixtures do not exercise (`alpha_prior`, `sd_scale`, `mask_thres`, `use_bcmatch` off / on,
 `mu_negctrl` fed from the negative-control fit, tiling `epsilon`): the CPU oracle against the reference's own model / guide
-programs, evaluated live through tests/refharness on the same screen and draws (float64; skipped without /root/reference)."""
+programs, evaluated live through tests/refharness on the same screen and draws (float64; skipped without BEAN_REFERENCE_ROOT)."""
 import copy
 from functools import partial
 

@@ -1,5 +1,5 @@
 """`prepare_bdata` (tests/support/prepare.py) against the reference's own function (bean/preprocessing/utils.py:24-67 +
-bean/qc/guide_qc.py:49-75, executed in place through tests/refharness where /root/reference is mounted) and against the
+bean/qc/guide_qc.py:49-75, executed in place through tests/refharness where BEAN_REFERENCE_ROOT is set) and against the
 behaviour it documents (portable checks)."""
 import os
 from types import SimpleNamespace

@@ -1,6 +1,6 @@
 """Caller-side helpers of `bean run` mirrored in crispr_bean_b200/run.py (`check_args`, `_get_guide_target_info`,
 `_get_guide_to_variant_df`, `_check_prior_params`) against the reference's own functions (bean/model/run.py:39-344,
-:479-542, executed in place through tests/refharness where /root/reference is mounted)."""
+:479-542, executed in place through tests/refharness where BEAN_REFERENCE_ROOT is set)."""
 import copy
 import pickle
 from types import SimpleNamespace

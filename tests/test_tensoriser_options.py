@@ -1,6 +1,6 @@
 """Tensoriser options the golden fixtures do not exercise (`shrink_alpha`, pre-fitted `popt` / `pi_popt`, `impute_pi_popt`,
 a replicate x guide outlier mask, masked samples, `use_const_pi`-free variants): the mirror's data classes against the
-reference's, built live through tests/refharness from the same screen (skipped where /root/reference is absent)."""
+reference's, built live through tests/refharness from the same screen (skipped without BEAN_REFERENCE_ROOT)."""
 import copy
 
 import numpy as np
