@@ -67,7 +67,7 @@ class BeanSviState(C.Structure):
         ("acc_k", C.c_void_p), ("noise_u", C.c_void_p), ("noise_m", C.c_void_p), ("noise_v", C.c_void_p),
         ("noise_grad", C.c_void_p),
         ("mu_prior_loc_v", C.c_void_p), ("mu_prior_scale_v", C.c_void_p), ("sd_prior_loc_v", C.c_void_p), ("sd_prior_scale_v", C.c_void_p),
-        ("pw", C.c_void_p), ("dconc", C.c_void_p),
+        ("pw", C.c_void_p), ("dconc", C.c_void_p), ("nonfinite_step", C.c_void_p),
     ]
 
 
@@ -91,7 +91,8 @@ class BeanAdamTensor(C.Structure):
 class BeanAdamArgs(C.Structure):
     _fields_ = [("n_tensors", C.c_int32), ("tensors", BeanAdamTensor * ADAM_MAX_TENSORS),
                 ("step_sizes", C.c_void_p), ("step", C.c_void_p), ("n_steps", C.c_int64),
-                ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double), ("clip", C.c_double)]
+                ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double), ("clip", C.c_double),
+                ("loss", C.c_void_p), ("nonfinite_step", C.c_void_p)]
 
 
 class BeanPiSitesArgs(C.Structure):
@@ -138,7 +139,7 @@ class BeanSurvivalState(C.Structure):
                 ("control_time", C.POINTER(C.c_double)), ("negctrl_loc", C.c_double), ("negctrl_scale", C.c_double),
                 ("log_obs", C.c_void_p), ("q0_u", C.c_void_p), ("q0_m", C.c_void_p), ("q0_v", C.c_void_p), ("q0_grad", C.c_void_p),
                 ("gamma", C.c_void_p * 2), ("sums", C.c_void_p * 2), ("abund_partial", C.c_void_p),
-                ("peers", C.POINTER(BeanPeerExchange))]
+                ("peers", C.POINTER(BeanPeerExchange)), ("nonfinite_step", C.c_void_p)]
 
 
 class BeanSurvivalNoise(C.Structure):
@@ -154,7 +155,8 @@ class BeanTilingState(C.Structure):
                 ("partial", C.c_void_p), ("counter", C.c_void_p), ("loss", C.c_void_p),
                 ("mu_prior_loc_v", C.c_void_p), ("mu_prior_scale_v", C.c_void_p), ("sd_prior_loc_v", C.c_void_p), ("sd_prior_scale_v", C.c_void_p),
                 ("epsilon", C.c_double), ("pi_tiny", C.c_double),
-                ("edit_sum", C.c_void_p), ("edit_iota", C.c_void_p), ("edit_term_weight", C.c_double)]
+                ("edit_sum", C.c_void_p), ("edit_iota", C.c_void_p), ("edit_term_weight", C.c_double),
+                ("nonfinite_step", C.c_void_p)]
 
 
 class BeanTilingNoise(C.Structure):
@@ -163,7 +165,7 @@ class BeanTilingNoise(C.Structure):
 
 SURV_PRIME_NONE, SURV_PRIME_AND_RUN, SURV_PRIME_ONLY = 0, 1, 2
 MODEL_NORMAL, MODEL_MIXTURE_NORMAL = 0, 1
-ABI_VERSION = 15  # include/bean_b200.h: BEAN_ABI_VERSION
+ABI_VERSION = 16  # include/bean_b200.h: BEAN_ABI_VERSION
 _GATHER = [C.POINTER(BeanAlleleMap), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
 _SCATTER = [C.POINTER(BeanAlleleMap), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
 
@@ -196,6 +198,7 @@ _PROTOTYPES = {
     "bean_peer_close": (C.c_int, [C.c_void_p]),
     "bean_peer_free": (C.c_int, [C.c_void_p]),
     "bean_peer_timeouts": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
+    "bean_peer_reset_flags": (C.c_int, [C.c_void_p]),
     "bean_svi_tiling_num_partials": (C.c_int, [C.c_int32, C.c_int32]),
     "bean_svi_tiling_run_f32": (C.c_int, [C.POINTER(BeanScreen), C.POINTER(BeanTilingState), C.POINTER(BeanSviConfig),
                                           C.POINTER(BeanTilingNoise), C.c_int32, C.c_int32, C.c_void_p]),

@@ -249,7 +249,8 @@ __device__ __forceinline__ double digamma_f64(double z) {
   // reference's pathwise Dirichlet derivative forms psi(a) + 1/a from it (model.py:937-938 through torch._dirichlet_grad), so
   // a differently ordered -- even a more accurate -- sum moves alpha_pi's gradient by ~2e-9.
   double result = 0.0, x = z;
-  while (x < 10.0) {
+  // bounded: a concentration is > 0 (at most 10 terms), but -inf or a huge negative argument would never reach 10
+  for (int k = 0; x < 10.0 && k < 64; ++k) {
     result -= 1.0 / x;
     x += 1.0;
   }

@@ -25,6 +25,8 @@ struct AdamParams {
   const long long* step;
   long long n_steps;
   real beta1, beta2, eps, clip;
+  const double* loss;   // loss[*step] or NULL
+  int* nonfinite;       // first non-finite step or NULL (BeanAdamArgs.nonfinite_step)
 };
 
 template <typename real>
@@ -33,14 +35,22 @@ __global__ void __launch_bounds__(ADAM_THREADS) clipped_adam_kernel(const AdamPa
   long long s = *p.step;
   s = s < 0 ? 0 : (s >= p.n_steps ? p.n_steps - 1 : s);
   const real step_size = real(p.step_sizes[s]);
+  real probe = real(0);  // NaN once a gradient was NaN / inf (g * 0): no predicate in the loop
   for (long long i = (long long)blockIdx.x * ADAM_THREADS + threadIdx.x; i < t.n; i += (long long)gridDim.x * ADAM_THREADS) {
     real g = t.grad[i];
+    probe += g * real(0);
     g = g < -p.clip ? -p.clip : (g > p.clip ? p.clip : g);  // elementwise clamp, not a norm clip
     const real m = p.beta1 * t.m[i] + (real(1) - p.beta1) * g;
     const real v = p.beta2 * t.v[i] + (real(1) - p.beta2) * g * g;
     t.m[i] = m;
     t.v[i] = v;
     t.theta[i] -= step_size * m / (sqrt(v) + p.eps);
+  }
+  if (p.nonfinite) {  // launch-uniform
+    bool bad = probe != probe;
+    if (p.loss && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) bad |= !isfinite(p.loss[s]);
+    const unsigned any = __ballot_sync(0xffffffffu, bad);
+    if (any != 0u && (int)(threadIdx.x & 31u) == __ffs(any) - 1 && *(volatile int*)p.nonfinite > (int)s) atomicMin(p.nonfinite, (int)s);
   }
 }
 
@@ -69,6 +79,8 @@ static int launch_adam(const BeanAdamArgs* a, void* stream) {
   p.step = reinterpret_cast<const long long*>(a->step);
   p.n_steps = a->n_steps;
   p.beta1 = real(a->beta1); p.beta2 = real(a->beta2); p.eps = real(a->eps); p.clip = real(a->clip);
+  p.loss = a->loss;
+  p.nonfinite = a->nonfinite_step;
   long long blocks = (n_max + ADAM_THREADS - 1) / ADAM_THREADS;
   if (blocks > 148 * 8) blocks = 148 * 8;  // grid-stride beyond one wave of 8 CTAs per SM
   const dim3 grid((unsigned)blocks, (unsigned)a->n_tensors);

@@ -52,6 +52,15 @@ int bean_peer_free(void* ptr) {
   return BEAN_OK;
 }
 
+// zero the step flags of this rank's own buffer, so that the next exchange waits for steps that are run again (a sharded fit
+// that is set back to an earlier step).  Synchronises; every rank must have finished writing to it before (host barrier).
+int bean_peer_reset_flags(void* own) {
+  BEAN_REQUIRE(own, BEAN_EINVAL, "own is NULL");
+  BEAN_CUDA(cudaMemset(static_cast<BeanPeerBuffer*>(own)->flag, 0, sizeof(static_cast<BeanPeerBuffer*>(own)->flag)));
+  BEAN_CUDA(cudaDeviceSynchronize());
+  return BEAN_OK;
+}
+
 // number of waits that gave up (a peer did not publish within BEAN_PEER_TIMEOUT_NS): 0 on a healthy run.  Synchronises.
 int bean_peer_timeouts(const void* own, unsigned long long* out) {
   BEAN_REQUIRE(own && out, BEAN_EINVAL, "own / out is NULL");

@@ -51,6 +51,7 @@ __global__ void __launch_bounds__(SVI_THREADS, ((SPLIT || !MIXTURE) && sizeof(re
   const int L = LFIX ? 2 : p.L;
   const real eps = real(1e-5);
   double elbo = 0.0;
+  bool bad = false;  // a ClippedAdam input of this thread was NaN / inf
   const int lane = threadIdx.x & 31;
   const unsigned wmask = __ballot_sync(0xffffffffu, g < p.G);  // lanes that own a guide: the warp-collective set below
   if (FAST) {
@@ -383,8 +384,8 @@ __global__ void __launch_bounds__(SVI_THREADS, ((SPLIT || !MIXTURE) && sizeof(re
         real th0 = p.alpha_u[2 * (size_t)g], th1 = p.alpha_u[2 * (size_t)g + 1];
         real m0 = p.alpha_m[2 * (size_t)g], m1 = p.alpha_m[2 * (size_t)g + 1];
         real v0 = p.alpha_v[2 * (size_t)g], v1 = p.alpha_v[2 * (size_t)g + 1];
-        clipped_adam(p, gl0, th0, m0, v0);
-        clipped_adam(p, gl1, th1, m1, v1);
+        clipped_adam(p, gl0, th0, m0, v0, bad);
+        clipped_adam(p, gl1, th1, m1, v1, bad);
         p.alpha_u[2 * (size_t)g] = th0; p.alpha_u[2 * (size_t)g + 1] = th1;
         p.alpha_m[2 * (size_t)g] = m0;  p.alpha_m[2 * (size_t)g + 1] = m1;
         p.alpha_v[2 * (size_t)g] = v0;  p.alpha_v[2 * (size_t)g + 1] = v1;
@@ -403,17 +404,18 @@ __global__ void __launch_bounds__(SVI_THREADS, ((SPLIT || !MIXTURE) && sizeof(re
         }
         if (p.apply_update) {
           real th = p.noise_u[g], m = p.noise_m[g], v = p.noise_v[g];
-          clipped_adam(p, gl, th, m, v);
+          clipped_adam(p, gl, th, m, v, bad);
           p.noise_u[g] = th; p.noise_m[g] = m; p.noise_v[g] = v;
           const size_t j = (size_t)p.G + g;
           th = p.noise_u[j]; m = p.noise_m[j]; v = p.noise_v[j];
-          clipped_adam(p, gs, th, m, v);
+          clipped_adam(p, gs, th, m, v, bad);
           p.noise_u[j] = th; p.noise_m[j] = m; p.noise_v[j] = v;
         }
       }
     }
     elbo = (double)elbo_g;
   }
+  if (MIXTURE && (!SPLIT || ACC)) note_nonfinite(p.nonfinite, p.step, 0xffffffffu, bad);
   const double tot = warp_sum(elbo);
   if ((threadIdx.x & 31) == 0) p.partial[(blockIdx.x * SVI_THREADS + threadIdx.x) / SVI_WARP] = tot;
 }
@@ -503,6 +505,7 @@ static int svi_run(const BeanScreen* s, const BeanSviState* state, const BeanSvi
   p.partial = state->partial;
   p.counter = state->counter;
   p.loss = state->loss;
+  p.nonfinite = state->nonfinite_step;
   p.n_partial_guide = (p.G + SVI_THREADS - 1) / SVI_THREADS * (SVI_THREADS / SVI_WARP);
   p.n_partial_var = (p.T + VAR_PER_CTA - 1) / VAR_PER_CTA;
   p.eps_mu = noise ? static_cast<const real*>(noise->eps_mu) : nullptr;

@@ -64,6 +64,7 @@ struct SviParams {
   double* partial;
   uint32_t* counter;
   double* loss;
+  int32_t* nonfinite;  // first non-finite step (include/bean_b200.h: BeanSviState.nonfinite_step) or NULL
   int n_partial_guide, n_partial_var;
   // injected noise (parity runs)
   const real* eps_mu;
@@ -109,10 +110,23 @@ struct SviParams {
   int dsd_times_sd;                     // d_guide's second row holds d/d(sd_allele) / sd_allele: multiply the sum by the edit's sd
 };
 
+// Step `step` is non-finite: keep the smallest such step in *word (atomicMin; the caller initialised it to INT32_MAX).  Skips
+// the atomic while the word already holds this step or an earlier one.
+__device__ __forceinline__ void record_nonfinite(int32_t* word, uint32_t step) {
+  if (*(volatile int32_t*)word > (int32_t)step) atomicMin(word, (int32_t)step);
+}
+// The same from a warp: every lane of `mask` calls with its own verdict, one lane of a warp that has any bad one records.
+__device__ __forceinline__ void note_nonfinite(int32_t* word, uint32_t step, unsigned mask, bool bad) {
+  if (word == nullptr) return;  // kernel-uniform
+  const unsigned any = __ballot_sync(mask, bad);
+  if (any != 0u && (int)(threadIdx.x & 31u) == __ffs(any) - 1) record_nonfinite(word, step);
+}
+
 // pyro.optim.ClippedAdam on one unconstrained scalar (SURVEY App. A.6); step_size carries
-// lr_t * sqrt(1 - beta2^t) / (1 - beta1^t).
+// lr_t * sqrt(1 - beta2^t) / (1 - beta1^t).  `bad` collects whether an input was NaN / inf (the clip below maps NaN to -clip).
 template <typename real>
-__device__ __forceinline__ void clipped_adam(const SviParams<real>& p, real grad, real& theta, real& m, real& v) {
+__device__ __forceinline__ void clipped_adam(const SviParams<real>& p, real grad, real& theta, real& m, real& v, bool& bad) {
+  bad |= !isfinite(grad);
   const real g = Num<real>::fmin(Num<real>::fmax(grad, -p.clip), p.clip);
   m = p.beta1 * m + (real(1) - p.beta1) * g;
   v = p.beta2 * v + (real(1) - p.beta2) * g * g;
@@ -144,7 +158,7 @@ __device__ __forceinline__ void variant_draw(const SviParams<real>& p, int v, re
 // concentration gradients -> log alpha_pi gradient -> ClippedAdam (alpha_pi is per guide)
 template <typename real>
 __device__ __forceinline__ void alpha_update(const SviParams<real>& p, int g, real al0, real al1, real pa0, real cm0, real cm1,
-                                             real dcm0, real dcm1, real dcg0, real dcg1) {
+                                             real dcm0, real dcm1, real dcg0, real dcg1, bool& bad) {
   const real eps = real(1e-5);
   const real asum = al0 + al1;
   // clamp(min) passes the gradient where its input >= 1e-5
@@ -162,8 +176,8 @@ __device__ __forceinline__ void alpha_update(const SviParams<real>& p, int g, re
     real th0 = p.alpha_u[2 * (size_t)g], th1 = p.alpha_u[2 * (size_t)g + 1];
     real m0 = p.alpha_m[2 * (size_t)g], m1 = p.alpha_m[2 * (size_t)g + 1];
     real v0 = p.alpha_v[2 * (size_t)g], v1 = p.alpha_v[2 * (size_t)g + 1];
-    clipped_adam(p, gl0, th0, m0, v0);
-    clipped_adam(p, gl1, th1, m1, v1);
+    clipped_adam(p, gl0, th0, m0, v0, bad);
+    clipped_adam(p, gl1, th1, m1, v1, bad);
     p.alpha_u[2 * (size_t)g] = th0; p.alpha_u[2 * (size_t)g + 1] = th1;
     p.alpha_m[2 * (size_t)g] = m0;  p.alpha_m[2 * (size_t)g + 1] = m1;
     p.alpha_v[2 * (size_t)g] = v0;  p.alpha_v[2 * (size_t)g + 1] = v1;
@@ -253,7 +267,9 @@ __global__ void __launch_bounds__(ALPHA_THREADS, BEAN_ALPHA_MIN_CTAS) svi_alpha_
     }
   }
   if (n_tail > 0) tail_queue_flush(tq, n_tail, wmask, lane, dcg0, dcg1);
-  alpha_update(p, g, al0, al1, pa0, cm0, cm1, dc.x, dc.y, dcg0, dcg1);
+  bool bad = false;
+  alpha_update(p, g, al0, al1, pa0, cm0, cm1, dc.x, dc.y, dcg0, dcg1, bad);
+  note_nonfinite(p.nonfinite, p.step, wmask, bad);
 }
 
 // This step's library-wide sums into shared memory: from `sums_cur` (single GPU, or the first step of a call: all-reduced by the
@@ -375,6 +391,7 @@ __global__ void __launch_bounds__(VAR_THREADS) svi_variant_kernel(const SviParam
   // this CTA's slice of the guide kernel's partials (fixed assignment: deterministic)
   double elbo = 0.0;
   for (int i = blockIdx.x * VAR_THREADS + threadIdx.x; i < p.n_partial_guide; i += gridDim.x * VAR_THREADS) elbo += p.partial[i];
+  bool bad = false;
   if (v < p.T) {
     real mu_t, sd_t, e_mu, e_sd, mu_scale, sd_scale, y;
     variant_draw(p, v, mu_t, sd_t, e_mu, e_sd, mu_scale, sd_scale, y);
@@ -420,7 +437,7 @@ __global__ void __launch_bounds__(VAR_THREADS) svi_variant_kernel(const SviParam
       if (p.var_grad) p.var_grad[i] = grad[k];
       if (p.apply_update) {
         real th = p.var_params[i], m = p.var_m[i], vv = p.var_v[i];
-        clipped_adam(p, grad[k], th, m, vv);
+        clipped_adam(p, grad[k], th, m, vv, bad);
         p.var_params[i] = th;
         p.var_m[i] = m;
         p.var_v[i] = vv;
@@ -440,6 +457,7 @@ __global__ void __launch_bounds__(VAR_THREADS) svi_variant_kernel(const SviParam
       __threadfence();
     }
   }
+  note_nonfinite(p.nonfinite, p.step, 0xffffffffu, bad);
   const double tot = block_sum(elbo, red);  // (its barriers also order the row written above before thread 0's fence)
   if (threadIdx.x == 0) {
     p.partial[p.n_partial_guide + blockIdx.x] = tot;
@@ -464,8 +482,10 @@ __global__ void __launch_bounds__(VAR_THREADS) svi_variant_kernel(const SviParam
     for (; i < n; i += VAR_THREADS) a0 += __ldcg(pv + i);
     const double all = block_sum((a0 + a1) + (a2 + a3), red);
     if (threadIdx.x == 0) {
-      p.loss[p.step] = -(all + p.ll_const);
+      const double loss = -(all + p.ll_const);
+      p.loss[p.step] = loss;
       *p.counter = 0u;
+      if (p.apply_update && p.nonfinite && !isfinite(loss)) record_nonfinite(p.nonfinite, p.step);
     }
     if (p.sums_next) {
       const double tot_j = column_sums(p.abund_partial + (size_t)p.n_abund_partial * C, M, C, 0, 1, s_cs);

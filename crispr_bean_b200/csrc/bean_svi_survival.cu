@@ -111,6 +111,7 @@ __global__ void __launch_bounds__(SVI_THREADS, sizeof(real) == 4 ? BEAN_SURV_MIN
   const real eps = real(1e-5);
   const bool owns = g < p.G;
   double elbo = 0.0;
+  bool bad = false;  // q0's ClippedAdam input was NaN / inf
   real c_next = real(0);
   __shared__ double s_sums[BEAN_PEER_MAX_VALS];
   load_library_sums(p, R + 1, s_sums);
@@ -324,12 +325,13 @@ __global__ void __launch_bounds__(SVI_THREADS, sizeof(real) == 4 ? BEAN_SURV_MIN
     c_next = c;
     if (p.apply_update) {
       real th = p.q0_u[g], m = p.q0_m[g], vv = p.q0_v[g];
-      clipped_adam(p, gq, th, m, vv);
+      clipped_adam(p, gq, th, m, vv, bad);
       p.q0_u[g] = th; p.q0_m[g] = m; p.q0_v[g] = vv;
       c_next = Num<real>::exp(th);
     }
     elbo = (double)elbo_g;
   }
+  note_nonfinite(p.nonfinite, p.step, 0xffffffffu, bad);
   const double tot = warp_sum(elbo);
   if ((threadIdx.x & 31) == 0) p.partial[(blockIdx.x * SVI_THREADS + threadIdx.x) / SVI_WARP] = tot;
   if (p.apply_update && p.gamma_next) draw_abundance(p, g, owns, c_next, p.step + 1u);
@@ -376,6 +378,7 @@ static int survival_run(const BeanScreen* s, const BeanSviState* state, const Be
   p.alpha_grad = static_cast<real*>(state->alpha_grad);
   p.pw = static_cast<real*>(state->pw); p.dconc = static_cast<real*>(state->dconc);
   p.partial = state->partial; p.counter = state->counter; p.loss = state->loss;
+  p.nonfinite = sv->nonfinite_step ? sv->nonfinite_step : state->nonfinite_step;
   p.n_partial_guide = (p.G + SVI_THREADS - 1) / SVI_THREADS * (SVI_THREADS / SVI_WARP);
   p.n_partial_var = (p.T + VAR_PER_CTA - 1) / VAR_PER_CTA;
   p.eps_mu = noise ? static_cast<const real*>(noise->eps_mu) : nullptr;

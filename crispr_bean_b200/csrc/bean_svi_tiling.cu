@@ -48,6 +48,7 @@ struct TilingParams {
   real* alpha_u; real* alpha_m; real* alpha_v; real* alpha_grad;  // [G][A]
   real* d_slot;              // [2][G * (A - 1)]: d ELBO / d mu_allele, (d ELBO / d sd_allele) / sd_allele
   double* partial;           // per-warp ELBO partials
+  int32_t* nonfinite;        // first non-finite step or NULL (BeanTilingState.nonfinite_step)
   const double* pi_in;       // [R][G][A] injected draws (parity) or NULL
   double* pi_out;
   double epsilon, prob_eps, pi_tiny;
@@ -297,6 +298,7 @@ __global__ void __launch_bounds__(TILING_MAX_REP_WARPS * 32) tiling_guide_kernel
   // ---- concentrations -> log alpha_pi (tiling_closed_form.py), ClippedAdam per existing allele
   const double dm = cm_live ? dcm : 0.0;
   const double sum_cg = warp_all_sum(has ? dcg * al : 0.0), sum_cm = warp_all_sum(has ? dm * (al + eps / A) : 0.0);
+  bool bad = false;
   if (has) {
     const double d_al = pa0 / (asum * asum) * (dcg * asum - sum_cg) + pa0 / S1 * (dm - sum_cm / S1);
     const real gl = exists ? real(-d_al * al) : real(0);
@@ -304,6 +306,7 @@ __global__ void __launch_bounds__(TILING_MAX_REP_WARPS * 32) tiling_guide_kernel
     if (p.alpha_grad) p.alpha_grad[i] = gl;
     if (p.apply_update) {
       real th = p.alpha_u[i], m = p.alpha_m[i], v = p.alpha_v[i];
+      bad = !isfinite(gl);
       const real gc = Num<real>::fmin(Num<real>::fmax(gl, -p.clip), p.clip);
       m = p.beta1 * m + (real(1) - p.beta1) * gc;
       v = p.beta2 * v + (real(1) - p.beta2) * gc * gc;
@@ -311,6 +314,7 @@ __global__ void __launch_bounds__(TILING_MAX_REP_WARPS * 32) tiling_guide_kernel
       p.alpha_u[i] = th; p.alpha_m[i] = m; p.alpha_v[i] = v;
     }
   }
+  note_nonfinite(p.nonfinite, p.step, 0xffffffffu, bad);
   const double tot = warp_all_sum(elbo);
   if (lane == 0) p.partial[g] = tot;
 }
@@ -346,7 +350,7 @@ static int tiling_run(const BeanScreen* s, const BeanTilingState* ts, const Bean
   v.var_params = static_cast<real*>(ts->edit_params); v.var_m = static_cast<real*>(ts->edit_m); v.var_v = static_cast<real*>(ts->edit_v);
   v.var_grad = static_cast<real*>(ts->edit_grad);
   v.d_guide = static_cast<real*>(ts->d_slot);
-  v.partial = ts->partial; v.counter = ts->counter; v.loss = ts->loss;
+  v.partial = ts->partial; v.counter = ts->counter; v.loss = ts->loss; v.nonfinite = ts->nonfinite_step;
   v.n_partial_guide = G;  // one ELBO partial per guide (warp)
   v.n_partial_var = (E + VAR_PER_CTA - 1) / VAR_PER_CTA;
   v.eps_mu = noise ? static_cast<const real*>(noise->eps_mu) : nullptr;
@@ -372,6 +376,7 @@ static int tiling_run(const BeanScreen* s, const BeanTilingState* ts, const Bean
   p.alpha_grad = static_cast<real*>(ts->alpha_grad);
   p.d_slot = static_cast<real*>(ts->d_slot);
   p.partial = ts->partial;
+  p.nonfinite = ts->nonfinite_step;
   p.pi_in = noise ? noise->pi : nullptr; p.pi_out = noise ? noise->pi_out : nullptr;
   p.epsilon = ts->epsilon > 0.0 ? ts->epsilon : 1e-5;
   p.prob_eps = cfg->prob_clamp_eps > 0.0 ? cfg->prob_clamp_eps : 2.220446049250313e-16;

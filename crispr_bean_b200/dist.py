@@ -68,18 +68,28 @@ def shard_data(data, rank: int, world: int):
 
 def run_sharded(make_engine: Callable, data, num_steps: int, rank: int, world: int,
                 all_reduce_sum: Optional[Callable] = None, all_gather: Optional[Callable] = None,
-                log_every: int = 100) -> Tuple[Dict[str, torch.Tensor], torch.Tensor]:
+                log_every: int = 100, all_reduce_min: Optional[Callable] = None) -> Tuple[Dict[str, torch.Tensor], torch.Tensor]:
     """SVI on this rank's shard; returns (global parameters, global loss per step).
 
-    make_engine(sub_data, guide_offset=..., variant_offset=...) -> object with .run(n), .losses(), .params().
-    `all_reduce_sum(tensor)` / `all_gather(tensor) -> list` default to torch.distributed when initialised.
+    make_engine(sub_data, guide_offset=..., variant_offset=...) -> an engine (.run(n), .losses(), .params(), .gradients(),
+    .nonfinite_step(), .snapshot(), .restore()).  `all_reduce_sum(tensor)` / `all_reduce_min(tensor)` /
+    `all_gather(tensor) -> list` default to torch.distributed when initialised.  A non-finite step on any rank raises
+    run.FitHalted on every rank, at the same step (the smallest over the ranks).
     """
     import torch.distributed as dist
+
+    from .halt import INT32_MAX
+    from .run import run_batches
 
     if all_reduce_sum is None:
         def all_reduce_sum(t):
             if world > 1:
                 dist.all_reduce(t)
+            return t
+    if all_reduce_min is None:
+        def all_reduce_min(t):
+            if world > 1:
+                dist.all_reduce(t, op=dist.ReduceOp.MIN)
             return t
     if all_gather is None:
         def all_gather(t):
@@ -96,21 +106,25 @@ def run_sharded(make_engine: Callable, data, num_steps: int, rank: int, world: i
 
     sub, off = shard_data(data, rank, world)
     eng = make_engine(sub, guide_offset=off["guide_offset"], variant_offset=off["variant_offset"])
-    done = 0
-    while done < num_steps:
-        n = min(log_every, num_steps - done)
-        eng.run(n)
-        done += n
-    # the one collective of the path: the per-step ELBO scalars, reduced once for the whole run
-    loss = all_reduce_sum(eng.losses().clone().to(_device_of(eng)))
-    params = {}
-    replicated = getattr(eng, "replicated_params", ())  # tiling: the per-edit parameters, identical on every rank
-    for k, v in eng.params().items():
-        if v.dim() == 0 or k in replicated:
-            params[k] = v
-        else:
-            params[k] = torch.cat(all_gather(v.contiguous()), dim=0)
-    return params, loss.cpu()
+
+    def agree(t):  # every rank stops at the first non-finite step of any rank
+        word = torch.tensor([INT32_MAX if t is None else t], dtype=torch.int64, device=_device_of(eng))
+        t = int(all_reduce_min(word).item())
+        return None if t == INT32_MAX else t
+
+    def collect(eng):
+        # the per-step ELBO scalars, reduced once for the whole run
+        loss = all_reduce_sum(eng.losses().clone().to(_device_of(eng)))
+        params = {}
+        replicated = getattr(eng, "replicated_params", ())  # tiling: the per-edit parameters, identical on every rank
+        for k, v in eng.params().items():
+            if v.dim() == 0 or k in replicated:
+                params[k] = v
+            else:
+                params[k] = torch.cat(all_gather(v.contiguous()), dim=0)
+        return params, loss.cpu()
+
+    return run_batches(eng, num_steps, log_every, collect=collect, agree=agree, rank=rank, log=False)
 
 
 def _device_of(eng):

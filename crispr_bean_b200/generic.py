@@ -21,6 +21,7 @@ import torch.distributions as tdist
 from . import _lib
 from ._lib import BeanError
 from .device_pack import DeviceScreen
+from .halt import NonfiniteWatch
 from .dirichlet import DirichletStream, dirichlet_rsample
 from .ll_function import count_log_likelihood
 from .latent_sites import LatentPrior, latent_sites
@@ -45,7 +46,7 @@ def _masked_sum(mask, lp):
     return torch.where(mask, lp, torch.zeros_like(lp)).sum()
 
 
-class AutogradSviEngine:
+class AutogradSviEngine(NonfiniteWatch):
     """Shared SVI plumbing of the models whose ELBO is assembled from torch CUDA ops around the C-ABI kernels:
     unconstrained parameters (positive ones as log), ClippedAdam (SURVEY App. A.6), device-side loss log."""
 
@@ -71,6 +72,7 @@ class AutogradSviEngine:
         t = torch.arange(1, max(num_steps, 1) + 1, dtype=torch.float64)
         self._step_sizes = (self.lr0 * self.lrd ** t * torch.sqrt(1 - 0.999 ** t) / (1 - 0.9 ** t)).to(self.device)
         self._t = torch.zeros(1, dtype=torch.int64, device=self.device)
+        self._nonfinite_ptr = self._init_nonfinite()
         # the `pi` draws: counter-based, keyed by (seed, global guide id, replicate, allele, device step counter)
         self.pi_stream = DirichletStream(seed, self._t, guide_offset=getattr(self, "guide_offset", 0), site=0)
         self._graph, self._graph_noise, self.use_graph = None, None, True
@@ -160,6 +162,7 @@ class AutogradSviEngine:
             args.n_tensors = n
             args.step_sizes, args.step, args.n_steps = self._step_sizes.data_ptr(), self._t.data_ptr(), self._step_sizes.numel()
             args.beta1, args.beta2, args.eps, args.clip = 0.9, 0.999, 1e-8, 10.0
+            args.loss, args.nonfinite_step = self.loss.data_ptr(), self._nonfinite_ptr  # loss[t] is written before this launch
             _lib.check(getattr(_lib.lib(), name)(args, stream), name)
 
     def _step_once(self, noise):
@@ -233,6 +236,15 @@ class AutogradSviEngine:
                 self._step_once(noise)
         self.step += n_steps
         return self.loss[self.step - n_steps:self.step]
+
+    def _snapshot_tensors(self):
+        return [*self.theta.values(), *self.m.values(), *self.v.values(), self._t]
+
+    def _snapshot_extra(self):
+        return {"gen": self.gen.get_state()}  # the captured step replays from the registered generator
+
+    def _restore_extra(self, snap):
+        self.gen.set_state(snap["gen"])
 
     def gradients(self, noise=None):
         for p in self.theta.values():

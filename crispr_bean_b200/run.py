@@ -6,8 +6,10 @@ bean/model/run.py:391-396, but the loop runs on the GPU with no host sync per st
 """
 from __future__ import annotations
 
+import pickle
 from functools import partial
 from logging import info
+from typing import Callable, Dict, List, Optional
 
 import torch
 
@@ -18,6 +20,72 @@ from .model import resolve, selection_of
 from .svi import SviEngine
 
 FUSED_MODELS = ("Normal", "ControlNormal", "MixtureNormal")
+DUMP_PATH = "tmp_result.pkl"  # where the reference's run_inference pickles the parameter store of a failed fit (run.py:381-390)
+
+
+class FitHalted(ValueError):
+    """SVI step `step` produced a NaN / inf loss or gradient, so the fit stopped before applying it, as the reference's fit does
+    under torch's anomaly mode.
+
+    step: the first non-finite step (0-based).
+    params: the parameters that step started from, {name: cpu tensor} -- exact, not the last batch boundary.
+    losses: the (finite) losses of steps 0 .. step - 1.
+    nonfinite: names among "loss" and the parameters whose value or gradient is non-finite at `params`.
+    The same parameters are pickled to ./tmp_result.pkl as {"param": params} (rank 0 only when sharded)."""
+
+    def __init__(self, step: int, params: Dict[str, torch.Tensor], losses: torch.Tensor, nonfinite: List[str]):
+        super().__init__(f"SVI step {step} is not finite ({', '.join(nonfinite) or 'no term isolated'}); "
+                         f"parameters of step {step} written to {DUMP_PATH}")
+        self.step, self.params, self.losses, self.nonfinite = step, params, losses, nonfinite
+
+
+def run_batches(eng, num_steps: int, log_every: int = 100, collect: Optional[Callable] = None,
+                agree: Optional[Callable] = None, rank: int = 0, log: bool = True):
+    """`num_steps` SVI steps of `eng` in batches of `log_every`; returns `collect(eng)` -> (params, losses).
+
+    After every batch the engine's first non-finite step is read (`agree` makes the ranks of a sharded fit agree on it: MIN).
+    Where there is one, the engine is set back to the start of the batch and re-runs the steps before it, and FitHalted is
+    raised with the parameters that step started from.  `collect` defaults to this engine's own (params, losses).  An engine
+    without `nonfinite_step` / `snapshot` / `restore` (a test double) is run without the check."""
+    if collect is None:
+        def collect(e):
+            return e.params(), e.losses()
+    watch = all(hasattr(eng, k) for k in ("nonfinite_step", "snapshot", "restore"))
+    done = 0
+    while done < num_steps:
+        n = min(log_every, num_steps - done)
+        snap = eng.snapshot() if watch else None
+        losses = eng.run(n)
+        if watch:
+            t = eng.nonfinite_step()
+            if agree is not None:
+                t = agree(t)
+            if t is not None:
+                _halt(eng, snap, t, done, collect, rank)
+        if log:
+            info(f"loss {losses[0].item()} @ iter {done}")  # reference prints every 100 steps (run.py:378-379)
+        done += n
+    return collect(eng)
+
+
+def _halt(eng, snap, t: int, batch_start: int, collect: Callable, rank: int):
+    eng.restore(snap)
+    if t > batch_start:
+        eng.run(t - batch_start)
+    grads = eng.gradients()  # step t's loss and gradient at theta_t (same counters as step t)
+    params, losses = collect(eng)
+    params = {k: v.detach().cpu() for k, v in params.items()}
+    own = eng.params()
+
+    def bad(x):
+        return x is not None and not bool(torch.isfinite(x).all())
+
+    nonfinite = ["loss"] if bad(grads["loss"]) else []
+    nonfinite += [k for k in own if bad(own[k]) or bad(grads.get(k))]
+    if rank == 0:
+        with open(DUMP_PATH, "wb") as f:
+            pickle.dump({"param": params}, f)
+    raise FitHalted(t, params, losses.detach().cpu()[:t], nonfinite)
 
 
 def make_engine(model, guide, data, initial_lr=0.01, gamma=0.1, num_steps=2000, device="cuda", dtype=torch.float32,
@@ -113,6 +181,9 @@ def run_inference(model, guide, data, initial_lr=0.01, gamma=0.1, num_steps=2000
                   dtype=torch.float32, seed=101, log_every=100):
     """Run SVI (one-particle Trace_ELBO + ClippedAdam, lr decaying by `gamma` over the run).
 
+    Raises FitHalted (a ValueError) at the first step whose loss or gradient is NaN / inf, with the parameters that step
+    started from, which are also pickled to ./tmp_result.pkl -- as the reference does (run.py:381-390).
+
     Same signature and return value as bean/model/run.py:347-396.  When torch.distributed is initialised with more than one
     rank (one process per GPU, e.g. under torchrun), every rank passes the SAME tensorised screen: the variants -- with all
     their guides -- are split over the ranks (`dist.shard_data`), each rank fits its block on its own GPU, the per-step ELBO
@@ -129,14 +200,8 @@ def run_inference(model, guide, data, initial_lr=0.01, gamma=0.1, num_steps=2000
         params, loss = run_sharded(make, data, num_steps, tdist.get_rank(), world, log_every=log_every)
         return params, {"loss": loss.tolist(), "params": {k: v.detach().cpu() for k, v in params.items()}}
     eng = make_engine(model, guide, data, initial_lr, gamma, num_steps, device, dtype, seed)
-    done = 0
-    while done < num_steps:
-        n = min(log_every, num_steps - done)
-        losses = eng.run(n)
-        info(f"loss {losses[0].item()} @ iter {done}")  # reference prints every 100 steps (run.py:378-379)
-        done += n
-    params = eng.params()
-    return params, {"loss": eng.losses().tolist(), "params": {k: v.detach().cpu() for k, v in params.items()}}
+    params, losses = run_batches(eng, num_steps, log_every)
+    return params, {"loss": losses.tolist(), "params": {k: v.detach().cpu() for k, v in params.items()}}
 
 
 def identify_model_guide(args):

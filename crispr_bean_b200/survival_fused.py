@@ -24,6 +24,7 @@ import torch
 
 from . import _lib
 from .device_pack import DeviceScreen, row_constants
+from .halt import NonfiniteWatch
 
 _RUN = {torch.float32: "bean_svi_survival_run_f32", torch.float64: "bean_svi_survival_run_f64"}
 
@@ -34,7 +35,7 @@ def _dist_active(group) -> bool:
     return dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
 
 
-class SurvivalFusedEngine:
+class SurvivalFusedEngine(NonfiniteWatch):
     def __init__(self, data, device="cuda", dtype=torch.float32, use_bcmatch: bool = True, num_steps: int = 2000,
                  initial_lr: float = 0.01, gamma: float = 0.1, seed: int = 101, alpha_prior: float = 1.0, mask_thres: int = 10,
                  prior_params: Optional[dict] = None, mu_negctrl=(0.0, 0.1), group=None, guide_offset: int = 0,
@@ -131,6 +132,7 @@ class SurvivalFusedEngine:
             s.mu_prior_loc_v = self._prior_v["mu_loc"].data_ptr()
         if "mu_scale" in self._prior_v:
             s.mu_prior_scale_v = self._prior_v["mu_scale"].data_ptr()
+        s.nonfinite_step = self._init_nonfinite()
         self.state = s
 
         v = _lib.BeanSurvivalState()
@@ -142,6 +144,7 @@ class SurvivalFusedEngine:
         v.gamma[0], v.gamma[1] = self.gamma[0].data_ptr(), self.gamma[1].data_ptr()
         v.sums[0], v.sums[1] = self.sums[0].data_ptr(), self.sums[1].data_ptr()
         v.abund_partial = self.abund_partial.data_ptr()
+        v.nonfinite_step = s.nonfinite_step
         self.surv = v
         self.peers, self._peers_tried = None, False  # opened by the first multi-step call of a sharded run (_open_peer_exchange)
 
@@ -210,6 +213,26 @@ class SurvivalFusedEngine:
                 self.peers = None
         except Exception:  # pragma: no cover  (interpreter shutdown)
             pass
+
+    def _snapshot_tensors(self):
+        # the abundance draws and library-wide sums of the next step are written by the step before it
+        return [self.var_params, self.var_m, self.var_v, self.alpha_u, self.alpha_m, self.alpha_v, self.q0_u, self.q0_m, self.q0_v,
+                *self.gamma, *self.sums]
+
+    def _snapshot_extra(self):
+        return {"primed": self._primed}
+
+    def _restore_extra(self, snap):
+        self._primed = snap["primed"]
+        if self.peers is not None:
+            # the exchange flags hold the step each rank last published and only grow: steps run again would not wait for
+            # their peers.  Every rank stops writing, then zeroes its own flags before any rank runs again.
+            import torch.distributed as dist
+
+            torch.cuda.synchronize(self.device)
+            dist.barrier(group=self.group)
+            _lib.check(self.lib.bean_peer_reset_flags(self._peer_own), "bean_peer_reset_flags")
+            dist.barrier(group=self.group)
 
     def _all_reduce(self, t):
         if _dist_active(self.group):

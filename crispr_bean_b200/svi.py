@@ -14,12 +14,13 @@ import torch
 
 from . import _lib
 from .device_pack import DeviceScreen, row_constants
+from .halt import NonfiniteWatch
 
 _RUN = {torch.float32: "bean_svi_run_f32", torch.float64: "bean_svi_run_f64"}
 VAR_PARAM_NAMES = ("mu_loc", "mu_scale", "sd_loc", "sd_scale")  # rows of var_params; scales stored as log
 
 
-class SviEngine:
+class SviEngine(NonfiniteWatch):
     """Parameters + optimiser state + the fused step for one (screen, model) pair on one GPU.
 
     model: "Normal" | "ControlNormal" | "MixtureNormal".  Parameter names, shapes and initial values
@@ -148,6 +149,7 @@ class SviEngine:
             s.acc_k = self.acc_k.data_ptr()
             s.noise_u, s.noise_m, s.noise_v = self.noise_u.data_ptr(), self.noise_m.data_ptr(), self.noise_v.data_ptr()
             s.noise_grad = self.noise_grad.data_ptr()
+        s.nonfinite_step = self._init_nonfinite()
         self.state = s
 
     # ---------------------------------------------------------------------------------------------
@@ -197,6 +199,14 @@ class SviEngine:
             self.step += n_steps
         self._keep = keep  # keep injected buffers alive until the stream has consumed them
         return self.loss[first:first + n_steps]
+
+    def _snapshot_tensors(self):
+        out = [self.var_params, self.var_m, self.var_v]
+        if self.mixture:
+            out += [self.alpha_u, self.alpha_m, self.alpha_v]
+        if self.acc:
+            out += [self.noise_u, self.noise_m, self.noise_v]
+        return out
 
     def gradients(self, noise=None) -> Dict[str, torch.Tensor]:
         """Loss and its gradient w.r.t. the unconstrained parameters at the current point (no update)."""

@@ -16,6 +16,7 @@ import torch
 
 from . import _lib
 from .device_pack import DeviceScreen, row_constants
+from .halt import NonfiniteWatch
 from .tiling import AlleleMap
 
 _RUN = {torch.float32: "bean_svi_tiling_run_f32", torch.float64: "bean_svi_tiling_run_f64"}
@@ -26,7 +27,7 @@ def supports(data, scale_by_accessibility: bool = False) -> bool:
     return (not scale_by_accessibility) and 2 <= int(data.n_max_alleles) <= MAX_ALLELES
 
 
-class TilingFusedEngine:
+class TilingFusedEngine(NonfiniteWatch):
     def __init__(self, data, device="cuda", dtype=torch.float32, use_bcmatch: bool = True, num_steps: int = 2000,
                  initial_lr: float = 0.01, gamma: float = 0.1, seed: int = 101, alpha_prior: float = 1.0, sd_scale: float = 0.01,
                  epsilon: float = 1e-5, prior_params: Optional[dict] = None, guide_offset: int = 0, group=None):
@@ -124,6 +125,7 @@ class TilingFusedEngine:
             self.edit_iota = torch.arange(E + 1, dtype=torch.int32, device=dev)
             s.edit_sum, s.edit_iota = self.edit_sum.data_ptr(), self.edit_iota.data_ptr()
             s.edit_term_weight = 1.0 if dist.get_rank(group) == 0 else 0.0  # the per-edit ELBO terms count once
+        s.nonfinite_step = self._init_nonfinite()
         self.state = s
 
     # ---------------------------------------------------------------------------------------------
@@ -179,6 +181,9 @@ class TilingFusedEngine:
             self.step += n_steps
         self._keep = keep
         return self.loss[first:first + n_steps]
+
+    def _snapshot_tensors(self):
+        return [self.edit_params, self.edit_m, self.edit_v, self.alpha_u, self.alpha_m, self.alpha_v]
 
     def gradients(self, noise=None) -> Dict[str, torch.Tensor]:
         """Loss and its gradient w.r.t. the unconstrained parameters at the current point (no update)."""

@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define BEAN_ABI_VERSION 15
+#define BEAN_ABI_VERSION 16
 
 enum {
   BEAN_OK = 0,
@@ -229,6 +229,10 @@ typedef struct BeanSviState {
      the alpha_pi update run in a second kernel that reads what the first one leaves here                          */
   void* pw;                      /* real [R][G][4]: (pi0, pi1, w0, w1) of every draw (replicate-major: coalesced)    */
   void* dconc;                   /* real [G][4]:    concentration gradients without the pathwise part               */
+  /* device i32 [1] or NULL (off): first non-finite step.  A step t that runs with apply_update = 1 and whose loss[t] or any
+     ClippedAdam input is NaN / inf does atomicMin(nonfinite_step, t); the caller initialises the word to INT32_MAX.  The update
+     of step t is still applied (the clip turns a NaN gradient into -clip): the caller discards what follows t.              */
+  int32_t* nonfinite_step;
 } BeanSviState;
 
 typedef struct BeanSviNoise {    /* all optional (NULL = draw with Philox) */
@@ -285,6 +289,7 @@ int bean_peer_open(const unsigned char* handle64, void** ptr);   /* map another 
 int bean_peer_close(void* ptr);
 int bean_peer_free(void* ptr);
 int bean_peer_timeouts(const void* own, unsigned long long* out);
+int bean_peer_reset_flags(void* own);                           /* zero own flags (a fit set back to an earlier step) */
 enum { BEAN_SURV_PRIME_NONE = 0, BEAN_SURV_PRIME_AND_RUN = 1, BEAN_SURV_PRIME_ONLY = 2 };
 typedef struct BeanSurvivalState {
   int32_t n_controls;            /* C: control conditions of the reporter Multinomial (BeanSviState.allele_counts is [R][C][G][2]) */
@@ -302,6 +307,7 @@ typedef struct BeanSurvivalState {
   double* sums[2];               /* f64 [R + 1] x 2: sum_g gamma[r][g] (r < R), sum_g q0[g] */
   double* abund_partial;         /* f64 [ceil(G / 128) * 4 + BEAN_SURV_FOLD_ROWS][R + 1] scratch */
   const BeanPeerExchange* peers; /* device-side exchange of `sums` between the ranks of a sharded run, or NULL */
+  int32_t* nonfinite_step;       /* as BeanSviState.nonfinite_step (q0 included); NULL: BeanSviState's is used */
 } BeanSurvivalState;
 typedef struct BeanSurvivalNoise { /* optional injected noise of the survival-only sites (parity runs) */
   const void* eps_negctrl;       /* real [G] standard-normal draw behind mu_negctrl */
@@ -376,6 +382,7 @@ typedef struct BeanTilingState {
   void* edit_sum;                /* real [2][E] or NULL (not sharded) */
   const int32_t* edit_iota;      /* i32 [E + 1] = 0, 1, ..., E (needed with edit_sum) */
   double edit_term_weight;
+  int32_t* nonfinite_step;       /* as BeanSviState.nonfinite_step (alpha_pi and the per-edit parameters) */
 } BeanTilingState;
 typedef struct BeanTilingNoise { /* all optional */
   const void* eps_mu;            /* real [E] */
@@ -504,6 +511,10 @@ typedef struct BeanAdamArgs {
   const int64_t* step;       /* device i64 [1]: 0-based index of this step */
   int64_t n_steps;
   double beta1, beta2, eps, clip;
+  /* first non-finite step, as BeanSviState.nonfinite_step: step *step is recorded when a gradient is NaN / inf or, with
+     `loss` set, when loss[*step] is (the caller writes it before this launch).  NULL: off                          */
+  const double* loss;        /* device f64 [n_steps] or NULL */
+  int32_t* nonfinite_step;   /* device i32 [1] or NULL */
 } BeanAdamArgs;
 int bean_clipped_adam_f32(const BeanAdamArgs* args, void* stream);
 int bean_clipped_adam_f64(const BeanAdamArgs* args, void* stream);
