@@ -165,7 +165,7 @@ class BeanTilingNoise(C.Structure):
 
 SURV_PRIME_NONE, SURV_PRIME_AND_RUN, SURV_PRIME_ONLY = 0, 1, 2
 MODEL_NORMAL, MODEL_MIXTURE_NORMAL = 0, 1
-ABI_VERSION = 16  # include/bean_b200.h: BEAN_ABI_VERSION
+ABI_VERSION = 17  # include/bean_b200.h: BEAN_ABI_VERSION
 _GATHER = [C.POINTER(BeanAlleleMap), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
 _SCATTER = [C.POINTER(BeanAlleleMap), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
 

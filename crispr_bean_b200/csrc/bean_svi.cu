@@ -10,8 +10,7 @@
 //       per warp; hands every draw (pi0, pi1) with its upstream weights to the alpha kernel.
 //   svi_alpha_kernel   (MixtureNormal) one thread per guide: the pathwise Dirichlet derivative of each draw
 //       (saddle-point pairs in double, the other regimes through a per-warp queue), the alpha_pi gradient AND
-//       its ClippedAdam update (alpha_pi is per-guide, so it never leaves the thread).  With no hand-over scratch
-//       (BeanSviState.pw == NULL) the guide kernel does this part itself.
+//       its ClippedAdam update (alpha_pi is per-guide, so it never leaves the thread).
 //   svi_variant_kernel 8 lanes per variant: segmented reduction of the per-guide gradients over the CSR
 //       variant range (no atomics; guides of a variant are contiguous, data_class.py:511-532), prior and
 //       entropy terms, ClippedAdam on (mu_loc, mu_scale, sd_loc, sd_scale), and -- in the last CTA to
@@ -20,18 +19,18 @@
 
 namespace bean {
 
-// SPLIT: the pathwise Dirichlet derivative and the alpha_pi update run in `svi_alpha_kernel` instead; this kernel hands
+// MixtureNormal: the pathwise Dirichlet derivative and the alpha_pi update run in `svi_alpha_kernel`; this kernel hands
 // over every draw with its upstream weights (16 B per replicate) and the rest of the concentration gradient.  Two small
-// instruction footprints instead of one large one (the I-cache is 32 KB per SM), at +0.26 GB of HBM traffic per step.
+// instruction footprints instead of one large one (the I-cache is 32 KB per SM), at +0.26 GB of HBM traffic per step:
+// 0.68 ms per step against 1.20 for the single kernel that did both (DESIGN section 5).
 //
 // FAST: the screen has exactly NB bins and no masked sample (sample_mask all ones: every screen without `bean qc` sample
 // drops).  The bin loops then carry no `b < B` predicates, the per-sample size factors come from a shared-memory table as
 // one 128-bit load per row instead of NB constant-bank loads with computed addresses, and the sample-mask multiplies are
 // gone -- together a third of the instructions of the get_alpha section (profiles/r2b_guide_source_top.txt: that section,
 // not the special functions, was the largest single block of the kernel after the round-2 instruction diet).
-template <typename real, int NB, bool MIXTURE, bool ACC, bool SPLIT, int FAST>
-__global__ void __launch_bounds__(SVI_THREADS, ((SPLIT || !MIXTURE) && sizeof(real) == 4) ? SVI_MIN_CTAS_SPLIT : SVI_MIN_CTAS) svi_guide_kernel(const SviParams<real> p) {
-  __shared__ TailQueue<real> tail_queues[SPLIT ? 1 : SVI_THREADS / SVI_WARP];
+template <typename real, int NB, bool MIXTURE, bool ACC, int FAST>
+__global__ void __launch_bounds__(SVI_THREADS, sizeof(real) == 4 ? SVI_GUIDE_MIN_CTAS_F32 : SVI_GUIDE_MIN_CTAS_F64) svi_guide_kernel(const SviParams<real> p) {
   __shared__ __align__(16) real s_sf[FAST ? BEAN_MAX_LAYERS * BEAN_MAX_RB : 1];  // [l][r][b] size factors
   // STAGE (float, 4 bins, mixture): the count rows and reporter counts of replicate r + 1 are copied global -> shared with
   // cp.async while replicate r is evaluated, double-buffered per thread; a row is then one LDS.128 (~30 cycles) instead of an
@@ -52,15 +51,11 @@ __global__ void __launch_bounds__(SVI_THREADS, ((SPLIT || !MIXTURE) && sizeof(re
   const real eps = real(1e-5);
   double elbo = 0.0;
   bool bad = false;  // a ClippedAdam input of this thread was NaN / inf
-  const int lane = threadIdx.x & 31;
-  const unsigned wmask = __ballot_sync(0xffffffffu, g < p.G);  // lanes that own a guide: the warp-collective set below
   if (FAST) {
     for (int i = threadIdx.x; i < L * R * NB; i += SVI_THREADS) s_sf[i] = p.t.sf[i / (R * NB)][i % (R * NB)];
     __syncthreads();
   }
   if (g < p.G) {
-    TailQueue<real>& tq = tail_queues[SPLIT ? 0 : threadIdx.x / SVI_WARP];
-    int n_tail = 0;
     const int v = p.guide_variant[g];
     real mu_t, sd_t, e_mu, e_sd, mu_scale, sd_scale, log_sd;
     variant_draw(p, v, mu_t, sd_t, e_mu, e_sd, mu_scale, sd_scale, log_sd);
@@ -312,7 +307,7 @@ __global__ void __launch_bounds__(SVI_THREADS, ((SPLIT || !MIXTURE) && sizeof(re
         // pathwise derivative of pi w.r.t. the guide concentration (torch _Dirichlet_backward)
         // evaluated in double even on the float path, as torch's CPU kernel does (accscalar_t = double):
         // the saddle-point branch cancels badly in float
-        if (SPLIT && sizeof(real) == 4) {
+        if (sizeof(real) == 4) {
           // go_a - (pi0 go0 + pi1 go1) without forming the weighted mean: with s = 1 - pi0 - pi1 (a few ulp: pi is a clamped,
           // rounded normalisation) it equals s go_a + pi_b (go_a - go_b), where nothing cancels -- as accurate as the double
           // evaluation rounded to float, in 6 FP32 instructions instead of 4 conversions + 4 FP64 operations
@@ -324,31 +319,14 @@ __global__ void __launch_bounds__(SVI_THREADS, ((SPLIT || !MIXTURE) && sizeof(re
         }
         const double gbar = (double)pi0 * (double)go0 + (double)pi1 * (double)go1;
         const double w0 = (double)go0 - gbar, w1 = (double)go1 - gbar;
-        if (SPLIT) {
-          typename Vec4<real>::type rec;
-          rec.x = pi0; rec.y = pi1; rec.z = real(w0); rec.w = real(w1);
-          reinterpret_cast<typename Vec4<real>::type*>(p.pw)[(size_t)r * p.G + g] = rec;  // replicate-major: a warp's stores coalesce
-          continue;
-        }
-        const bool saddle = dirichlet_pair_is_saddle((double)pi0, (double)pi1, (double)cg[0], (double)cg[1]);
-        if (saddle) {
-          double dg0, dg1;
-          dirichlet_pair_saddle_f64((double)pi0, (double)pi1, (double)cg[0], (double)cg[1], dg0, dg1);
-          dcg[0] += real(dg0 * w0);
-          dcg[1] += real(dg1 * w1);
-        }
-        // every other regime is deferred: queued per warp, evaluated with all lanes busy (bean_rng.cuh, TailQueue)
-        n_tail = tail_queue_push(tq, n_tail, wmask, lane, !saddle, pi0, pi1, cg[0], cg[1], real(w0), real(w1));
-        if (n_tail >= 32) {
-          tail_queue_flush(tq, n_tail, wmask, lane, dcg[0], dcg[1]);
-          n_tail = 0;
-        }
+        typename Vec4<real>::type rec;
+        rec.x = pi0; rec.y = pi1; rec.z = real(w0); rec.w = real(w1);
+        reinterpret_cast<typename Vec4<real>::type*>(p.pw)[(size_t)r * p.G + g] = rec;  // replicate-major: a warp's stores coalesce
       } else {
 #pragma unroll
         for (int b = 0; b < NB; ++b) dP[b] += de[b];
       }
     }
-    if (MIXTURE && !SPLIT && n_tail > 0) tail_queue_flush(tq, n_tail, wmask, lane, dcg[0], dcg[1]);
     // per-guide gradient w.r.t. the edited allele's (mu, sd_targets); reduced per variant by the next kernel
     real dmu = real(0), dsg = real(0);
 #pragma unroll
@@ -363,33 +341,10 @@ __global__ void __launch_bounds__(SVI_THREADS, ((SPLIT || !MIXTURE) && sizeof(re
     if (p.sd_is_sqrt) dsg *= real(0.5) / sigma;
     p.d_guide[g] = dmu;
     p.d_guide[(size_t)p.G + g] = dsg;
-    if (MIXTURE && SPLIT) {
+    if (MIXTURE) {
       typename Vec4<real>::type rec;
       rec.x = dcm[0]; rec.y = dcm[1]; rec.z = dcg[0]; rec.w = dcg[1];
       reinterpret_cast<typename Vec4<real>::type*>(p.dconc)[g] = rec;
-    }
-    if (MIXTURE && !SPLIT) {
-      // concentration -> log alpha_pi; clamp(min) passes the gradient where its input >= 1e-5
-      const real dC0 = dcm[0] + (cm[0] >= eps ? dcg[0] : real(0));
-      const real dC1 = dcm[1] + (cm[1] >= eps ? dcg[1] : real(0));
-      const real k = pa0 / (asum * asum);
-      const real dal0 = k * (dC0 * (asum - al[0]) - dC1 * al[1]);
-      const real dal1 = k * (dC1 * (asum - al[1]) - dC0 * al[0]);
-      const real gl0 = -dal0 * al[0], gl1 = -dal1 * al[1];  // loss = -ELBO, unconstrained (log) space
-      if (p.alpha_grad) {
-        p.alpha_grad[2 * (size_t)g] = gl0;
-        p.alpha_grad[2 * (size_t)g + 1] = gl1;
-      }
-      if (p.apply_update) {
-        real th0 = p.alpha_u[2 * (size_t)g], th1 = p.alpha_u[2 * (size_t)g + 1];
-        real m0 = p.alpha_m[2 * (size_t)g], m1 = p.alpha_m[2 * (size_t)g + 1];
-        real v0 = p.alpha_v[2 * (size_t)g], v1 = p.alpha_v[2 * (size_t)g + 1];
-        clipped_adam(p, gl0, th0, m0, v0, bad);
-        clipped_adam(p, gl1, th1, m1, v1, bad);
-        p.alpha_u[2 * (size_t)g] = th0; p.alpha_u[2 * (size_t)g + 1] = th1;
-        p.alpha_m[2 * (size_t)g] = m0;  p.alpha_m[2 * (size_t)g + 1] = m1;
-        p.alpha_v[2 * (size_t)g] = v0;  p.alpha_v[2 * (size_t)g + 1] = v1;
-      }
     }
     if (acc) {
       // logit_pi_noise site: model Normal(0, 0.655); guide Normal(noise_loc, noise_scale) or the prior itself
@@ -415,30 +370,29 @@ __global__ void __launch_bounds__(SVI_THREADS, ((SPLIT || !MIXTURE) && sizeof(re
     }
     elbo = (double)elbo_g;
   }
-  if (MIXTURE && (!SPLIT || ACC)) note_nonfinite(p.nonfinite, p.step, 0xffffffffu, bad);
+  if (MIXTURE && ACC) note_nonfinite(p.nonfinite, p.step, 0xffffffffu, bad);
   const double tot = warp_sum(elbo);
   if ((threadIdx.x & 31) == 0) p.partial[(blockIdx.x * SVI_THREADS + threadIdx.x) / SVI_WARP] = tot;
 }
 
-template <typename real, bool MIXTURE, bool ACC, bool SPLIT>
+template <typename real, bool MIXTURE, bool ACC>
 static void launch_guide(const SviParams<real>& p, cudaStream_t st, bool guide, bool alpha, bool fast) {
   const int grid = (p.G + SVI_THREADS - 1) / SVI_THREADS;
-  constexpr bool HAS_FAST = true;
   if (!guide) {
-  } else if (HAS_FAST && fast && p.B == 4 && p.L == 2)
-    launch_after(svi_guide_kernel<real, 4, MIXTURE, ACC, SPLIT, 2>, grid, SVI_THREADS, st, p);
-  else if (HAS_FAST && fast && p.B == 4)
-    launch_after(svi_guide_kernel<real, 4, MIXTURE, ACC, SPLIT, 1>, grid, SVI_THREADS, st, p);
-  else if (HAS_FAST && fast && p.B == 5)
-    launch_after(svi_guide_kernel<real, 5, MIXTURE, ACC, SPLIT, 1>, grid, SVI_THREADS, st, p);
+  } else if (fast && p.B == 4 && p.L == 2)
+    launch_after(svi_guide_kernel<real, 4, MIXTURE, ACC, 2>, grid, SVI_THREADS, st, p);
+  else if (fast && p.B == 4)
+    launch_after(svi_guide_kernel<real, 4, MIXTURE, ACC, 1>, grid, SVI_THREADS, st, p);
+  else if (fast && p.B == 5)
+    launch_after(svi_guide_kernel<real, 5, MIXTURE, ACC, 1>, grid, SVI_THREADS, st, p);
   else if (p.B <= 4)
-    launch_after(svi_guide_kernel<real, 4, MIXTURE, ACC, SPLIT, 0>, grid, SVI_THREADS, st, p);
+    launch_after(svi_guide_kernel<real, 4, MIXTURE, ACC, 0>, grid, SVI_THREADS, st, p);
   else if (p.B == 5)
-    launch_after(svi_guide_kernel<real, 5, MIXTURE, ACC, SPLIT, 0>, grid, SVI_THREADS, st, p);
+    launch_after(svi_guide_kernel<real, 5, MIXTURE, ACC, 0>, grid, SVI_THREADS, st, p);
   else
-    launch_after(svi_guide_kernel<real, BEAN_MAX_BINS, MIXTURE, ACC, SPLIT, 0>, grid, SVI_THREADS, st, p);
+    launch_after(svi_guide_kernel<real, BEAN_MAX_BINS, MIXTURE, ACC, 0>, grid, SVI_THREADS, st, p);
   // (one thread per (guide, replicate) with a shuffle reduction was tried for this kernel: 0.42 vs 0.27 ms)
-  if (MIXTURE && SPLIT && alpha) launch_after(svi_alpha_kernel<real>, (p.G + ALPHA_THREADS - 1) / ALPHA_THREADS, ALPHA_THREADS, st, p);
+  if (MIXTURE && alpha) launch_after(svi_alpha_kernel<real>, (p.G + ALPHA_THREADS - 1) / ALPHA_THREADS, ALPHA_THREADS, st, p);
 }
 
 template <typename real>
@@ -457,26 +411,18 @@ static int svi_run(const BeanScreen* s, const BeanSviState* state, const BeanSvi
   if (mix) {
     BEAN_REQUIRE(state->allele_counts && state->pi_a0, BEAN_EINVAL, "MixtureNormal needs allele_counts / pi_a0");
     BEAN_REQUIRE(state->alpha_u && state->alpha_m && state->alpha_v, BEAN_EINVAL, "MixtureNormal needs alpha_u / alpha_m / alpha_v");
+    BEAN_REQUIRE(state->pw && state->dconc, BEAN_EINVAL, "MixtureNormal needs the hand-over scratch pw / dconc");
+    BEAN_REQUIRE(aligned16(state->pw) && aligned16(state->dconc), BEAN_EALIGN, "pw / dconc are not 16-byte aligned");
   }
   if (mix && state->acc_k && cfg->fit_noise)
     BEAN_REQUIRE(state->noise_u && state->noise_m && state->noise_v, BEAN_EINVAL, "fit_noise needs noise_u / noise_m / noise_v");
-  BEAN_REQUIRE(first_step >= 0 && n_steps >= 0, BEAN_EINVAL, "first_step / n_steps must be >= 0");
-  BEAN_REQUIRE(first_step + n_steps <= state->loss_capacity, BEAN_EINVAL, "loss buffer too small: %d + %d > %d", first_step,
-               n_steps, state->loss_capacity);
-  if (noise && (noise->eps_mu || noise->eps_sd))
-    BEAN_REQUIRE(noise->eps_mu && noise->eps_sd, BEAN_EINVAL, "eps_mu and eps_sd must be injected together");
+  if ((rc = check_step_range(first_step, n_steps, state->loss_capacity)) != BEAN_OK) return rc;
+  if (noise && (rc = check_eps_pair(noise->eps_mu, noise->eps_sd)) != BEAN_OK) return rc;
 
   SviParams<real> p{};  // zero: every optional pointer NULL, every mode flag off
-  p.G = s->n_guides; p.R = s->n_reps; p.B = s->n_bins; p.L = s->n_layers; p.T = state->n_variants;
-  p.mixture = mix; p.sd_is_sqrt = cfg->sd_is_sqrt; p.mu_prior_normal = cfg->mu_prior_normal; p.apply_update = cfg->apply_update;
-  p.seed = cfg->seed;
-  philox_round_keys(p.seed, p.rk);
-  p.guide_offset = cfg->guide_offset;
-  p.variant_offset = cfg->variant_offset;
-  p.mask_thres = real(s->mask_thres);
-  p.x = static_cast<const real*>(s->x);
-  p.a0 = static_cast<const real*>(s->a0);
-  p.row_mask = s->row_mask;
+  fill_common(p, s, cfg);
+  p.T = state->n_variants;
+  p.mixture = mix; p.sd_is_sqrt = cfg->sd_is_sqrt; p.has_sd = 1;
   p.guide_variant = state->guide_variant;
   p.variant_ptr = state->variant_ptr;
   p.allele_counts = static_cast<const real*>(state->allele_counts);
@@ -493,15 +439,11 @@ static int svi_run(const BeanScreen* s, const BeanSviState* state, const BeanSvi
   p.noise_v = static_cast<real*>(state->noise_v);
   p.noise_grad = static_cast<real*>(state->noise_grad);
   p.fit_noise = cfg->fit_noise;
-  p.has_sd = 1;
-  p.gather_idx = nullptr; p.dsd_times_sd = 0;
-  p.sums_next = nullptr; p.abund_partial = nullptr; p.n_abund_partial = 0; p.peer_world = 0;
   p.d_guide = static_cast<real*>(state->d_guide);
   p.var_grad = static_cast<real*>(state->var_grad);
   p.alpha_grad = static_cast<real*>(state->alpha_grad);
   p.pw = static_cast<real*>(state->pw);
   p.dconc = static_cast<real*>(state->dconc);
-  if (p.pw) BEAN_REQUIRE(aligned16(p.pw) && aligned16(p.dconc), BEAN_EALIGN, "pw / dconc are not 16-byte aligned");
   p.partial = state->partial;
   p.counter = state->counter;
   p.loss = state->loss;
@@ -514,16 +456,10 @@ static int svi_run(const BeanScreen* s, const BeanSviState* state, const BeanSvi
   p.eps_noise = noise ? static_cast<const real*>(noise->eps_noise) : nullptr;
   p.eps_out = noise ? static_cast<real*>(noise->eps_out) : nullptr;
   p.pi_out = noise ? static_cast<real*>(noise->pi_out) : nullptr;
-  p.mu_prior_loc = real(cfg->mu_prior_loc); p.mu_prior_scale = real(cfg->mu_prior_scale);
-  p.sd_prior_loc = real(cfg->sd_prior_loc); p.sd_prior_scale = real(cfg->sd_prior_scale);
   p.mu_prior_loc_v = static_cast<const real*>(state->mu_prior_loc_v);
   p.mu_prior_scale_v = static_cast<const real*>(state->mu_prior_scale_v);
   p.sd_prior_loc_v = static_cast<const real*>(state->sd_prior_loc_v);
   p.sd_prior_scale_v = static_cast<const real*>(state->sd_prior_scale_v);
-  p.beta1 = real(cfg->beta1); p.beta2 = real(cfg->beta2); p.adam_eps = real(cfg->adam_eps); p.clip = real(cfg->clip);
-  p.ll_const = cfg->ll_const;
-  p.prob_eps = cfg->prob_clamp_eps > 0.0 ? real(cfg->prob_clamp_eps) : Lim<real>::eps();
-  fill_tables(s, p.t);
   for (int b = 0; b < BEAN_MAX_BINS; ++b) {
     double m = 0.0;
     if (b < s->n_bins) {  // wild-type allele N(0, 1): Phi(t_u) - Phi(t_l), as get_std_normal_prob does in float64
@@ -538,20 +474,14 @@ static int svi_run(const BeanScreen* s, const BeanSviState* state, const BeanSvi
   bool fast = (s->n_bins == 4 || s->n_bins == 5) && !cfg->force_generic;
   for (int i = 0; i < s->n_reps * s->n_bins; ++i) fast = fast && s->sample_mask[i] == 1.0;
   for (int i = 0; i < n_steps; ++i) {
-    const int t = first_step + i;  // 0-based step; ClippedAdam's state["step"] = t + 1
+    const int t = first_step + i;
     p.step = (uint32_t)t;
-    const double lr = cfg->lr0 * pow(cfg->lrd, (double)(t + 1));
-    p.step_size = real(lr * sqrt(1.0 - pow(cfg->beta2, (double)(t + 1))) / (1.0 - pow(cfg->beta1, (double)(t + 1))));
-    // phases: 0 = the whole step; otherwise a bit mask (1 guide kernel, 2 variant kernel, 4 alpha kernel) so that a
-    // benchmark can time each kernel alone with CUDA events
-    const int ph = cfg->phases == 0 ? 7 : cfg->phases;
+    p.step_size = adam_step_size<real>(cfg, t);
+    const int ph = step_phases(cfg);
     const bool do_guide = ph & 1, do_alpha = ph & 4;
-    if (do_guide || do_alpha) {
-      const bool split = mix && p.pw != nullptr && p.dconc != nullptr;
-      if (mix && p.acc_k) { if (split) launch_guide<real, true, true, true>(p, st, do_guide, do_alpha, fast); else launch_guide<real, true, true, false>(p, st, do_guide, false, fast); }
-      else if (mix) { if (split) launch_guide<real, true, false, true>(p, st, do_guide, do_alpha, fast); else launch_guide<real, true, false, false>(p, st, do_guide, false, fast); }
-      else launch_guide<real, false, false, false>(p, st, do_guide, false, fast);
-    }
+    if (mix && p.acc_k) launch_guide<real, true, true>(p, st, do_guide, do_alpha, fast);
+    else if (mix) launch_guide<real, true, false>(p, st, do_guide, do_alpha, fast);
+    else launch_guide<real, false, false>(p, st, do_guide, false, fast);
     if (ph & 2) launch_after(svi_variant_kernel<real>, p.n_partial_var, VAR_THREADS, st, p);
   }
   BEAN_CUDA(cudaPeekAtLastError());

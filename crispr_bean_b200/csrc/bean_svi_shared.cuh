@@ -12,11 +12,11 @@
 namespace bean {
 
 constexpr int SVI_THREADS = 128;
-constexpr int SVI_MIN_CTAS = 4;        // fused guide step: <= 128 registers, 16 warps/SM (more CTAs measured +-2 %)
+constexpr int SVI_GUIDE_MIN_CTAS_F64 = 4;  // double guide kernels: <= 128 registers, 16 warps/SM (more CTAs measured +-2 %)
 #ifndef BEAN_GUIDE_MIN_CTAS
 #define BEAN_GUIDE_MIN_CTAS 7  // with the cp.async-staged rows: 6: 0.4243, 7: 0.4132, 8: 0.4235 ms per launch at c5 (profiles/r2h_phase_times.jsonl)
 #endif
-constexpr int SVI_MIN_CTAS_SPLIT = BEAN_GUIDE_MIN_CTAS;  // split guide step and the Normal models: 72 registers, 28 warps/SM
+constexpr int SVI_GUIDE_MIN_CTAS_F32 = BEAN_GUIDE_MIN_CTAS;  // float guide kernels: 72 registers, 28 warps/SM
                                        // (MixtureNormal 4: 1.17, 6: 1.11, 8: 1.08 ms/step; Normal 4: 0.64, 8: 0.58; final kernel 7: 0.650, 8: 0.640 ms)
 // ELBO partials are per WARP (no CTA barrier: per-guide cost varies with the Dirichlet-gradient regime of its draws,
 // so the warps of a CTA finish far apart).  1-warp CTAs were tried and were 4 % slower.
@@ -59,8 +59,8 @@ struct SviParams {
   real* d_guide;
   real* var_grad;
   real* alpha_grad;
-  real* pw;      // split path: [R][G][4] = (pi0, pi1, w0, w1) of every draw, written by the guide kernel
-  real* dconc;   // split path: [G][4]    = (dcm0, dcm1, dcg0, dcg1) without the pathwise part
+  real* pw;      // MixtureNormal: [R][G][4] = (pi0, pi1, w0, w1) of every draw, written by the guide kernel
+  real* dconc;   // MixtureNormal: [G][4]    = (dcm0, dcm1, dcg0, dcg1) without the pathwise part
   double* partial;
   uint32_t* counter;
   double* loss;
@@ -215,7 +215,52 @@ static inline void launch_after(Kernel kernel, int grid, int block, cudaStream_t
 #endif
 }
 
-// Second half of the split guide step: pathwise Dirichlet derivative of every draw (saddle-point pairs in place, the other
+// ---- host side of the run functions (bean_svi.cu, bean_svi_survival.cu, bean_svi_tiling.cu)
+
+inline int check_step_range(int32_t first_step, int32_t n_steps, int32_t capacity) {
+  BEAN_REQUIRE(first_step >= 0 && n_steps >= 0 && first_step + n_steps <= capacity, BEAN_EINVAL, "bad step range %d + %d (capacity %d)",
+               first_step, n_steps, capacity);
+  return BEAN_OK;
+}
+inline int check_eps_pair(const void* eps_mu, const void* eps_sd) {
+  if (eps_mu || eps_sd) BEAN_REQUIRE(eps_mu && eps_sd, BEAN_EINVAL, "eps_mu and eps_sd must be injected together");
+  return BEAN_OK;
+}
+
+// ClippedAdam's step size of 0-based step t (state["step"] = t + 1): lr_t * sqrt(1 - beta2^(t+1)) / (1 - beta1^(t+1))
+template <typename real>
+inline real adam_step_size(const BeanSviConfig* cfg, int t) {
+  const double lr = cfg->lr0 * pow(cfg->lrd, (double)(t + 1));
+  return real(lr * sqrt(1.0 - pow(cfg->beta2, (double)(t + 1))) / (1.0 - pow(cfg->beta1, (double)(t + 1))));
+}
+
+// BeanSviConfig.phases: 0 = the whole step; otherwise a bit mask (1 guide kernel, 2 variant kernel, 4 alpha kernel) so that a
+// benchmark can time each kernel alone with CUDA events
+inline int step_phases(const BeanSviConfig* cfg) { return cfg->phases == 0 ? 7 : cfg->phases; }
+
+// What every step kind takes from the screen and the config: sizes, counters, the count rows, priors and optimiser constants.
+// The caller sets T, has_sd and the buffers of its step.
+template <typename real>
+inline void fill_common(SviParams<real>& p, const BeanScreen* s, const BeanSviConfig* cfg) {
+  p.G = s->n_guides; p.R = s->n_reps; p.B = s->n_bins; p.L = s->n_layers;
+  p.mu_prior_normal = cfg->mu_prior_normal; p.apply_update = cfg->apply_update;
+  p.seed = cfg->seed;
+  philox_round_keys(p.seed, p.rk);
+  p.guide_offset = cfg->guide_offset;
+  p.variant_offset = cfg->variant_offset;
+  p.mask_thres = real(s->mask_thres);
+  p.x = static_cast<const real*>(s->x);
+  p.a0 = static_cast<const real*>(s->a0);
+  p.row_mask = s->row_mask;
+  p.mu_prior_loc = real(cfg->mu_prior_loc); p.mu_prior_scale = real(cfg->mu_prior_scale);
+  p.sd_prior_loc = real(cfg->sd_prior_loc); p.sd_prior_scale = real(cfg->sd_prior_scale);
+  p.beta1 = real(cfg->beta1); p.beta2 = real(cfg->beta2); p.adam_eps = real(cfg->adam_eps); p.clip = real(cfg->clip);
+  p.ll_const = cfg->ll_const;
+  p.prob_eps = cfg->prob_clamp_eps > 0.0 ? real(cfg->prob_clamp_eps) : Lim<real>::eps();
+  fill_tables(s, p.t);
+}
+
+// Second half of the MixtureNormal guide step: pathwise Dirichlet derivative of every draw (saddle-point pairs in place, the other
 // regimes through the per-warp queue), alpha_pi gradient and its ClippedAdam update.  One thread per guide.
 // one warp per CTA: the work per draw differs by regime, and small CTAs hand their SM slot on as soon as their own 32 guides are
 // done (128 / 64 / 32 threads: 0.161 / 0.160 / 0.155 ms at c5, 0.057 / 0.055 / 0.054 at a quarter of it; profiles/r2p_variants.jsonl)

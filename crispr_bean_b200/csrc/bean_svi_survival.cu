@@ -355,19 +355,14 @@ static int survival_run(const BeanScreen* s, const BeanSviState* state, const Be
                BEAN_SURV_MAX_CTRL);
   BEAN_REQUIRE(sv->control_time != nullptr, BEAN_EINVAL, "control_time is NULL");
   BEAN_REQUIRE(aligned16(state->pw) && aligned16(state->dconc), BEAN_EALIGN, "pw / dconc are not 16-byte aligned");
-  BEAN_REQUIRE(first_step >= 0 && n_steps >= 0 && first_step + n_steps <= state->loss_capacity, BEAN_EINVAL, "bad step range %d + %d (capacity %d)",
-               first_step, n_steps, state->loss_capacity);
+  if ((rc = check_step_range(first_step, n_steps, state->loss_capacity)) != BEAN_OK) return rc;
 
   SviParams<real> p{};  // zero: every optional pointer NULL, every mode flag off
   memset(&p, 0, sizeof(p));
-  p.G = s->n_guides; p.R = s->n_reps; p.B = s->n_bins; p.L = s->n_layers; p.T = state->n_variants;
-  p.mixture = 1; p.has_sd = 0; p.mu_prior_normal = cfg->mu_prior_normal; p.apply_update = cfg->apply_update;
-  p.seed = cfg->seed; p.guide_offset = cfg->guide_offset; p.variant_offset = cfg->variant_offset;
-  philox_round_keys(p.seed, p.rk);
-  p.mask_thres = real(s->mask_thres);
-  p.x = static_cast<const real*>(s->x);
-  p.a0 = static_cast<const real*>(s->a0);
-  p.row_mask = s->row_mask;
+  fill_common(p, s, cfg);
+  p.T = state->n_variants;
+  p.mixture = 1; p.has_sd = 0;
+  p.sd_prior_loc = real(0); p.sd_prior_scale = real(1);  // no sd_targets site: the per-variant kernel's sd terms stay inert
   p.guide_variant = state->guide_variant; p.variant_ptr = state->variant_ptr;
   p.allele_counts = static_cast<const real*>(state->allele_counts);
   p.pi_a0 = static_cast<const real*>(state->pi_a0);
@@ -388,14 +383,8 @@ static int survival_run(const BeanScreen* s, const BeanSviState* state, const Be
   p.pi_out = noise ? static_cast<real*>(noise->pi_out) : nullptr;
   p.eps_negctrl = snoise ? static_cast<const real*>(snoise->eps_negctrl) : nullptr;
   p.q0_in = snoise ? static_cast<const real*>(snoise->q0) : nullptr;
-  p.mu_prior_loc = real(cfg->mu_prior_loc); p.mu_prior_scale = real(cfg->mu_prior_scale);
-  p.sd_prior_loc = real(0); p.sd_prior_scale = real(1);
   p.mu_prior_loc_v = static_cast<const real*>(state->mu_prior_loc_v);
   p.mu_prior_scale_v = static_cast<const real*>(state->mu_prior_scale_v);
-  p.beta1 = real(cfg->beta1); p.beta2 = real(cfg->beta2); p.adam_eps = real(cfg->adam_eps); p.clip = real(cfg->clip);
-  p.ll_const = cfg->ll_const;
-  p.prob_eps = cfg->prob_clamp_eps > 0.0 ? real(cfg->prob_clamp_eps) : Lim<real>::eps();
-  fill_tables(s, p.t);
   p.n_ctrl = sv->n_controls;
   for (int c = 0; c < BEAN_SURV_MAX_CTRL; ++c) p.t_ctrl[c] = c < sv->n_controls ? real(sv->control_time[c]) : real(0);
   p.negctrl_loc = real(sv->negctrl_loc); p.negctrl_scale = real(sv->negctrl_scale);
@@ -424,8 +413,7 @@ static int survival_run(const BeanScreen* s, const BeanSviState* state, const Be
     const int t = first_step + i;
     p.step = (uint32_t)t;
     p.peer_consume = i > 0 ? 1 : 0;
-    const double lr = cfg->lr0 * pow(cfg->lrd, (double)(t + 1));
-    p.step_size = real(lr * sqrt(1.0 - pow(cfg->beta2, (double)(t + 1))) / (1.0 - pow(cfg->beta1, (double)(t + 1))));
+    p.step_size = adam_step_size<real>(cfg, t);
     // the abundance draw of step t lives in buffer t & 1 (written by the step before, or primed here)
     const int cur = t & 1;
     if (sv->prime != BEAN_SURV_PRIME_NONE && i == 0) {
@@ -439,9 +427,7 @@ static int survival_run(const BeanScreen* s, const BeanSviState* state, const Be
     p.sums_cur = sv->sums[cur];
     p.gamma_next = cfg->apply_update ? static_cast<real*>(sv->gamma[cur ^ 1]) : nullptr;
     p.sums_next = cfg->apply_update ? sv->sums[cur ^ 1] : nullptr;
-    // phases: 0 = the whole step; otherwise a bit mask (1 guide kernel, 2 variant kernel, 4 alpha kernel) so that a benchmark
-    // can time each kernel alone with CUDA events
-    const int ph = cfg->phases == 0 ? 7 : cfg->phases;
+    const int ph = step_phases(cfg);
     if (ph & 1) {
       if (p.B == 3)
         launch_after(surv_guide_kernel<real, 3, true>, grid, SVI_THREADS, st, p);

@@ -334,18 +334,17 @@ static int tiling_run(const BeanScreen* s, const BeanTilingState* ts, const Bean
   BEAN_REQUIRE(ts->allele_mask && ts->pi_a0 && ts->counts, BEAN_EINVAL, "allele_mask / pi_a0 / counts must be non-NULL");
   BEAN_REQUIRE(ts->edit_params && ts->edit_m && ts->edit_v && ts->alpha_u && ts->alpha_m && ts->alpha_v, BEAN_EINVAL, "parameter buffers must be non-NULL");
   BEAN_REQUIRE(ts->mu_e && ts->sd_e && ts->d_slot && ts->partial && ts->counter && ts->loss, BEAN_EINVAL, "scratch buffers must be non-NULL");
-  BEAN_REQUIRE(first_step >= 0 && n_steps >= 0 && first_step + n_steps <= ts->loss_capacity, BEAN_EINVAL, "bad step range %d + %d (capacity %d)",
-               first_step, n_steps, ts->loss_capacity);
-  if (noise && (noise->eps_mu || noise->eps_sd)) BEAN_REQUIRE(noise->eps_mu && noise->eps_sd, BEAN_EINVAL, "eps_mu and eps_sd must be injected together");
+  if ((rc = check_step_range(first_step, n_steps, ts->loss_capacity)) != BEAN_OK) return rc;
+  if (noise && (rc = check_eps_pair(noise->eps_mu, noise->eps_sd)) != BEAN_OK) return rc;
 
   const int G = s->n_guides;
   const int n_slots = G * (A - 1);
   // ---- the per-edit kernels: SviParams with the edits as variants
   SviParams<real> v;
   memset(&v, 0, sizeof(v));
-  v.G = n_slots; v.R = s->n_reps; v.B = s->n_bins; v.L = s->n_layers; v.T = E;
-  v.has_sd = 1; v.mu_prior_normal = cfg->mu_prior_normal; v.apply_update = cfg->apply_update;
-  v.seed = cfg->seed; v.variant_offset = cfg->variant_offset;
+  fill_common(v, s, cfg);
+  v.G = n_slots; v.T = E;
+  v.has_sd = 1;
   v.variant_ptr = ts->map->edit_ptr; v.gather_idx = ts->map->edit_slot; v.dsd_times_sd = 1;
   v.var_params = static_cast<real*>(ts->edit_params); v.var_m = static_cast<real*>(ts->edit_m); v.var_v = static_cast<real*>(ts->edit_v);
   v.var_grad = static_cast<real*>(ts->edit_grad);
@@ -356,12 +355,8 @@ static int tiling_run(const BeanScreen* s, const BeanTilingState* ts, const Bean
   v.eps_mu = noise ? static_cast<const real*>(noise->eps_mu) : nullptr;
   v.eps_sd = noise ? static_cast<const real*>(noise->eps_sd) : nullptr;
   v.eps_out = noise ? static_cast<real*>(noise->eps_out) : nullptr;
-  v.mu_prior_loc = real(cfg->mu_prior_loc); v.mu_prior_scale = real(cfg->mu_prior_scale);
-  v.sd_prior_loc = real(cfg->sd_prior_loc); v.sd_prior_scale = real(cfg->sd_prior_scale);
   v.mu_prior_loc_v = static_cast<const real*>(ts->mu_prior_loc_v); v.mu_prior_scale_v = static_cast<const real*>(ts->mu_prior_scale_v);
   v.sd_prior_loc_v = static_cast<const real*>(ts->sd_prior_loc_v); v.sd_prior_scale_v = static_cast<const real*>(ts->sd_prior_scale_v);
-  v.beta1 = real(cfg->beta1); v.beta2 = real(cfg->beta2); v.adam_eps = real(cfg->adam_eps); v.clip = real(cfg->clip);
-  v.ll_const = cfg->ll_const;
   // ---- the per-guide kernel
   TilingParams<real> p;
   memset(&p, 0, sizeof(p));
@@ -410,8 +405,7 @@ static int tiling_run(const BeanScreen* s, const BeanTilingState* ts, const Bean
   for (int i = 0; i < n_steps; ++i) {
     const int t = first_step + i;
     v.step = u.step = p.step = (uint32_t)t;
-    const double lr = cfg->lr0 * pow(cfg->lrd, (double)(t + 1));
-    v.step_size = u.step_size = p.step_size = real(lr * sqrt(1.0 - pow(cfg->beta2, (double)(t + 1))) / (1.0 - pow(cfg->beta1, (double)(t + 1))));
+    v.step_size = u.step_size = p.step_size = adam_step_size<real>(cfg, t);
     if (sharded && cfg->phases == 2) {
       launch_after(svi_variant_kernel<real>, u.n_partial_var, VAR_THREADS, st, u);
       continue;

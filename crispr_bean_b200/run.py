@@ -100,62 +100,47 @@ def make_engine(model, guide, data, initial_lr=0.01, gamma=0.1, num_steps=2000, 
         raise BeanError("run_inference needs a CUDA device: crispr_bean_b200 has no CPU fallback")
     if selection_of(model) != selection_of(guide):
         raise ValueError("model and guide belong to different selections (sorting vs survival)")
+    use_bcmatch = mkw.get("use_bcmatch", True)
+    use_bcmatch = True if isinstance(use_bcmatch, tuple) else bool(use_bcmatch)  # the reference passes a 1-tuple (App. B2)
+    kw = dict(device=device, dtype=dtype, num_steps=num_steps, initial_lr=initial_lr, gamma=gamma, seed=seed,
+              prior_params=mkw.get("prior_params"))
+    alpha_prior, sd_scale = float(mkw.get("alpha_prior", 1.0)), float(mkw.get("sd_scale", 0.01))
+    mask_thres, epsilon = int(mkw.get("mask_thres", 10)), float(mkw.get("epsilon", 1e-5))
+    scale_by_acc = bool(mkw.get("scale_by_accessibility", False))
+    fit_noise = bool(gkw.get("fit_noise", False))  # only the GUIDE's fit_noise matters: the model is never given it (App. B3)
     if selection_of(model) == "survival":
         from .survival import SurvivalSviEngine
 
-        use_bcmatch = mkw.get("use_bcmatch", True)
-        use_bcmatch = True if isinstance(use_bcmatch, tuple) else bool(use_bcmatch)  # App. B2
         extra = {}
         if name in ("MixtureNormal", "MultiMixtureNormal"):
-            extra = dict(mu_negctrl=mkw["mu_negctrl"], scale_by_accessibility=bool(mkw.get("scale_by_accessibility", False)),
-                         fit_noise=bool(gkw.get("fit_noise", False)))
+            extra = dict(mu_negctrl=mkw["mu_negctrl"], scale_by_accessibility=scale_by_acc, fit_noise=fit_noise)
         if name == "MultiMixtureNormal":
-            extra["epsilon"] = float(mkw.get("epsilon", 1e-5))
-        if name == "MixtureNormal" and not extra["scale_by_accessibility"]:
+            extra["epsilon"] = epsilon
+        if name == "MixtureNormal" and not scale_by_acc:
             from .survival_fused import SurvivalFusedEngine  # the whole step as three CUDA kernels
 
-            return SurvivalFusedEngine(data, device=device, dtype=dtype, use_bcmatch=use_bcmatch, num_steps=num_steps,
-                                       initial_lr=initial_lr, gamma=gamma, seed=seed, alpha_prior=float(mkw.get("alpha_prior", 1.0)),
-                                       mask_thres=int(mkw.get("mask_thres", 10)), prior_params=mkw.get("prior_params"),
-                                       mu_negctrl=mkw["mu_negctrl"], guide_offset=guide_offset, variant_offset=variant_offset)
-        return SurvivalSviEngine(data, name, device=device, dtype=dtype, use_bcmatch=use_bcmatch, num_steps=num_steps,
-                                 initial_lr=initial_lr, gamma=gamma, seed=seed, alpha_prior=float(mkw.get("alpha_prior", 1.0)),
-                                 mask_thres=int(mkw.get("mask_thres", 10)), prior_params=mkw.get("prior_params"),
-                                 guide_offset=guide_offset, **extra)
+            return SurvivalFusedEngine(data, use_bcmatch=use_bcmatch, alpha_prior=alpha_prior, mask_thres=mask_thres,
+                                       mu_negctrl=mkw["mu_negctrl"], guide_offset=guide_offset, variant_offset=variant_offset, **kw)
+        return SurvivalSviEngine(data, name, use_bcmatch=use_bcmatch, alpha_prior=alpha_prior, mask_thres=mask_thres,
+                                 guide_offset=guide_offset, **extra, **kw)
     if name == "MultiMixtureNormal":
         from .generic import TilingSviEngine
         from . import tiling_fused
 
-        if tiling_fused.supports(data, bool(mkw.get("scale_by_accessibility", False))):  # <= 32 alleles per guide, no --scale-by-acc
-            return tiling_fused.TilingFusedEngine(data, device=device, dtype=dtype, use_bcmatch=True, num_steps=num_steps,
-                                                  initial_lr=initial_lr, gamma=gamma, seed=seed, alpha_prior=float(mkw.get("alpha_prior", 1.0)),
-                                                  sd_scale=float(mkw.get("sd_scale", 0.01)), epsilon=float(mkw.get("epsilon", 1e-5)),
-                                                  prior_params=mkw.get("prior_params"), guide_offset=guide_offset)
-        return TilingSviEngine(data, device=device, dtype=dtype, use_bcmatch=True, num_steps=num_steps, initial_lr=initial_lr,
-                               gamma=gamma, seed=seed, alpha_prior=float(mkw.get("alpha_prior", 1.0)),
-                               sd_scale=float(mkw.get("sd_scale", 0.01)), epsilon=float(mkw.get("epsilon", 1e-5)),
-                               prior_params=mkw.get("prior_params"),
-                               scale_by_accessibility=bool(mkw.get("scale_by_accessibility", False)),
-                               fit_noise=bool(gkw.get("fit_noise", False)))
+        if tiling_fused.supports(data, scale_by_acc):  # <= 32 alleles per guide, no --scale-by-acc
+            return tiling_fused.TilingFusedEngine(data, use_bcmatch=True, alpha_prior=alpha_prior, sd_scale=sd_scale, epsilon=epsilon,
+                                                  guide_offset=guide_offset, **kw)
+        return TilingSviEngine(data, use_bcmatch=True, alpha_prior=alpha_prior, sd_scale=sd_scale, epsilon=epsilon,
+                               scale_by_accessibility=scale_by_acc, fit_noise=fit_noise, **kw)
     if name == "Normal" and getattr(data, "sample_covariates", None) is not None:
         from .generic import CovariateNormalEngine  # replicate-specific means: not in the fused kernel
 
-        return CovariateNormalEngine(data, device=device, dtype=dtype, use_bcmatch=bool(mkw.get("use_bcmatch", True)),
-                                     num_steps=num_steps, initial_lr=initial_lr, gamma=gamma, seed=seed,
-                                     sd_scale=float(mkw.get("sd_scale", 0.01)), mask_thres=int(mkw.get("mask_thres", 10)),
-                                     prior_params=mkw.get("prior_params"))
+        return CovariateNormalEngine(data, use_bcmatch=use_bcmatch, sd_scale=sd_scale, mask_thres=mask_thres, **kw)
     if name not in FUSED_MODELS:
         raise NotImplementedError(f"model {name} is not built yet")
-    use_bcmatch = mkw.get("use_bcmatch", True)
-    if isinstance(use_bcmatch, tuple):  # reference passes the 1-tuple (not args.ignore_bcmatch,): always truthy (App. B2)
-        use_bcmatch = True
-    return SviEngine(
-        data, name, device=device, dtype=dtype, use_bcmatch=use_bcmatch, num_steps=num_steps, initial_lr=initial_lr,
-        gamma=gamma, seed=seed, alpha_prior=float(mkw.get("alpha_prior", 1.0)), sd_scale=float(mkw.get("sd_scale", 0.01)),
-        mask_thres=int(mkw.get("mask_thres", 10)), prior_params=mkw.get("prior_params"),
-        scale_by_accessibility=bool(mkw.get("scale_by_accessibility", False)),
-        # only the GUIDE's fit_noise matters: the model is never given it (SURVEY App. B3)
-        fit_noise=bool(gkw.get("fit_noise", False)), guide_offset=guide_offset, variant_offset=variant_offset)
+    return SviEngine(data, name, use_bcmatch=use_bcmatch, alpha_prior=alpha_prior, sd_scale=sd_scale, mask_thres=mask_thres,
+                     scale_by_accessibility=scale_by_acc, fit_noise=fit_noise, guide_offset=guide_offset,
+                     variant_offset=variant_offset, **kw)
 
 
 def shards_over_ranks(model, data) -> bool:

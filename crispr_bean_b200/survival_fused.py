@@ -24,18 +24,12 @@ import torch
 
 from . import _lib
 from .device_pack import DeviceScreen, row_constants
-from .halt import NonfiniteWatch
+from .fused import FusedEngine, dist_active, set_prior_pointers, svi_config
 
 _RUN = {torch.float32: "bean_svi_survival_run_f32", torch.float64: "bean_svi_survival_run_f64"}
 
 
-def _dist_active(group) -> bool:
-    import torch.distributed as dist
-
-    return dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
-
-
-class SurvivalFusedEngine(NonfiniteWatch):
+class SurvivalFusedEngine(FusedEngine):
     def __init__(self, data, device="cuda", dtype=torch.float32, use_bcmatch: bool = True, num_steps: int = 2000,
                  initial_lr: float = 0.01, gamma: float = 0.1, seed: int = 101, alpha_prior: float = 1.0, mask_thres: int = 10,
                  prior_params: Optional[dict] = None, mu_negctrl=(0.0, 0.1), group=None, guide_offset: int = 0,
@@ -44,10 +38,9 @@ class SurvivalFusedEngine(NonfiniteWatch):
             raise ValueError("SurvivalFusedEngine needs a *SurvivalScreenData object")
         if not torch.cuda.is_available():
             raise _lib.BeanError("SurvivalFusedEngine needs a CUDA device: there is no CPU fallback")
-        self.lib = _lib.lib()
-        self.model, self.dtype, self.device, self.group = "MixtureNormal", dtype, torch.device(device), group
-        self.num_steps = int(num_steps)
-        self.sharded = _dist_active(group)
+        self._setup(device, dtype, num_steps)
+        self.model, self.group = "MixtureNormal", group
+        self.sharded = dist_active(group)
         use_bcmatch = bool(use_bcmatch) and getattr(data, "X_bcmatch_masked", None) is not None
         self.screen = screen or DeviceScreen(data, self.device, dtype=dtype, use_bcmatch=use_bcmatch, mask_thres=mask_thres)
         G, R, T = self.screen.n_guides, self.screen.n_reps, int(data.n_targets)
@@ -81,42 +74,17 @@ class SurvivalFusedEngine(NonfiniteWatch):
         n_partial = self.lib.bean_svi_num_partials(G, T)
         self.partial = torch.zeros(n_partial, dtype=torch.float64, device=dev)
         self.abund_partial = torch.zeros(((G + 127) // 128 * 4 + _lib.SURV_FOLD_ROWS, R + 1), dtype=torch.float64, device=dev)
-        self.counter = torch.zeros(1, dtype=torch.int32, device=dev)
-        self.loss = torch.zeros(max(self.num_steps, 1) + 1, dtype=torch.float64, device=dev)
         self.pw, self.dconc = torch.empty((R, G, 4), **kw), torch.empty((G, 4), **kw)
-        self.step, self._primed = 0, False
+        self._primed = False
         # data-only parts of the ELBO: Dirichlet-Multinomial rows (DeviceScreen) + the reporter Multinomial's coefficient
         mconst, _ = row_constants(self.allele_counts, with_xlogx=False)  # (R, C, G)
         ll_const = self.screen.ll_const + float((mconst * (self.screen.row_mask != 0).unsqueeze(1)).sum())
 
-        c = _lib.BeanSviConfig()
-        c.model, c.sd_is_sqrt, c.apply_update, c.fit_noise = _lib.MODEL_MIXTURE_NORMAL, 0, 1, 0
-        c.mu_prior_normal, c.mu_prior_loc, c.mu_prior_scale = 0, 0.0, 1.0
-        self._prior_v = {}
-        if prior_params and ("mu_loc" in prior_params or "mu_scale" in prior_params):
-            c.mu_prior_normal = 1
-            for key in ("mu_loc", "mu_scale"):
-                if key in prior_params:
-                    val = prior_params[key]
-                    if torch.is_tensor(val) and val.numel() > 1:
-                        if val.numel() != T:
-                            raise ValueError(f"prior_params[{key!r}] has {val.numel()} entries for {T} variants")
-                        self._prior_v[key] = val.detach().reshape(-1).to(**kw).contiguous()
-                    else:
-                        setattr(c, f"mu_prior_{key[3:]}", float(val))
-        c.sd_prior_loc, c.sd_prior_scale = 0.0, 1.0
-        c.lr0, c.lrd = float(initial_lr), float(gamma) ** (1.0 / max(self.num_steps, 1))
-        c.beta1, c.beta2, c.adam_eps, c.clip = 0.9, 0.999, 1e-8, 10.0
-        c.ll_const, c.seed = ll_const, int(seed)
-        # the reference evaluates pi exp(mu t_c) in the promoted dtype of (pi_a0, control_timepoint): float64 out of its data
-        # class even on the float32 path, and torch's Multinomial clamps probabilities at the eps of THAT dtype
-        pa0 = getattr(data, "pi_a0", None)
-        ref_dtype = dtype
-        for t in (pa0, data.control_timepoint):
-            if torch.is_tensor(t):
-                ref_dtype = torch.promote_types(ref_dtype, t.dtype)
-        c.prob_clamp_eps = float(torch.finfo(ref_dtype).eps)
-        c.guide_offset, c.variant_offset = int(guide_offset), int(variant_offset)
+        c, self._prior_v = svi_config(lr=initial_lr, gamma=gamma, num_steps=self.num_steps, seed=seed, ll_const=ll_const,
+                                      guide_offset=guide_offset, variant_offset=variant_offset, sd_priors=False,
+                                      prior_params=prior_params, n_variants=T, device=dev, dtype=dtype,
+                                      pi_a0=getattr(data, "pi_a0", None), control_timepoint=data.control_timepoint, promote=True)
+        c.sd_is_sqrt, c.fit_noise = 0, 0
         self.cfg = c
 
         s = _lib.BeanSviState()
@@ -128,10 +96,7 @@ class SurvivalFusedEngine(NonfiniteWatch):
         s.d_guide = self.d_guide.data_ptr()
         s.partial, s.counter, s.loss = self.partial.data_ptr(), self.counter.data_ptr(), self.loss.data_ptr()
         s.pw, s.dconc = self.pw.data_ptr(), self.dconc.data_ptr()
-        if "mu_loc" in self._prior_v:
-            s.mu_prior_loc_v = self._prior_v["mu_loc"].data_ptr()
-        if "mu_scale" in self._prior_v:
-            s.mu_prior_scale_v = self._prior_v["mu_scale"].data_ptr()
+        set_prior_pointers(s, self._prior_v)
         s.nonfinite_step = self._init_nonfinite()
         self.state = s
 
@@ -235,7 +200,7 @@ class SurvivalFusedEngine(NonfiniteWatch):
             dist.barrier(group=self.group)
 
     def _all_reduce(self, t):
-        if _dist_active(self.group):
+        if dist_active(self.group):
             import torch.distributed as dist
 
             dist.all_reduce(t, group=self.group)
@@ -244,82 +209,60 @@ class SurvivalFusedEngine(NonfiniteWatch):
     def _noise_structs(self, noise):
         if noise is None:
             return None, None, ()
-        kw = dict(device=self.device, dtype=self.dtype)
         n, sn, keep = _lib.BeanSviNoise(), _lib.BeanSurvivalNoise(), []
-
-        def put(struct, field, tensor, shape):
-            t = tensor.to(**kw).contiguous()
-            assert tuple(t.shape) == shape, (field, tuple(t.shape), shape)
-            setattr(struct, field, t.data_ptr())
-            keep.append(t)
-
         if "eps_mu" in noise:
-            put(n, "eps_mu", noise["eps_mu"].reshape(-1), (self.T,))
+            self._put(keep, n, "eps_mu", noise["eps_mu"].reshape(-1), (self.T,))
         if "pi" in noise:
             pi = noise["pi"]
             if pi.dim() == 4:  # reference layout (R, 1, G, 2) -> kernel layout (G, R, 2)
                 pi = pi[:, 0].permute(1, 0, 2)
-            put(n, "pi", pi, (self.G, self.R, 2))
+            self._put(keep, n, "pi", pi, (self.G, self.R, 2))
         if "eps_negctrl" in noise:
-            put(sn, "eps_negctrl", noise["eps_negctrl"].reshape(-1), (self.G,))
+            self._put(keep, sn, "eps_negctrl", noise["eps_negctrl"].reshape(-1), (self.G,))
         if "q0" in noise:
-            put(sn, "q0", noise["q0"], (self.R, self.G))
+            self._put(keep, sn, "q0", noise["q0"], (self.R, self.G))
         return n, sn, keep
 
-    def _launch(self, first, n, noise_structs, prime):
-        n_struct, sn_struct, keep = noise_structs
+    def _call(self, first, n, noise_structs, prime):
+        n_struct, sn_struct, _ = noise_structs
         self.surv.prime = prime
         stream = torch.cuda.current_stream(self.device).cuda_stream
         rc = getattr(self.lib, _RUN[self.dtype])(self.screen.c, self.state, self.surv, self.cfg, n_struct, sn_struct, first, n, stream)
         _lib.check(rc, _RUN[self.dtype])
-        self._keep = keep
 
-    def run(self, n_steps: int, noise: Optional[Dict[str, torch.Tensor]] = None, apply_update: bool = True):
-        """Advance `n_steps` SVI steps (asynchronously); injected `noise` applies to every one of them."""
-        if self.step + n_steps > self.loss.numel() - (1 if apply_update else 0):
-            raise ValueError("loss buffer exhausted: construct the engine with a larger num_steps")
+    def _launch(self, first, n_steps, noise, apply_update):
         ns = self._noise_structs(noise)
-        self.cfg.apply_update = 1 if apply_update else 0
-        first = self.step
         self.surv.peers = None
         if not self.sharded:
-            self._launch(first, n_steps, ns, _lib.SURV_PRIME_NONE if self._primed else _lib.SURV_PRIME_AND_RUN)
+            self._call(first, n_steps, ns, _lib.SURV_PRIME_NONE if self._primed else _lib.SURV_PRIME_AND_RUN)
         elif apply_update and self.cfg.phases == 0 and n_steps > 1 and self._peer_exchange() is not None:
             # device-side exchange: the ranks trade their R + 1 partial sums through peer memory inside the kernels, the host
             # all-reduces only the sums the NEXT call starts from
             if not self._primed:
-                self._launch(first, 1, ns, _lib.SURV_PRIME_ONLY)
+                self._call(first, 1, ns, _lib.SURV_PRIME_ONLY)
                 self._all_reduce(self.sums[first & 1])
                 self._primed = True
             self.surv.peers = C.pointer(self.peers)
-            self._launch(first, n_steps, ns, _lib.SURV_PRIME_NONE)
+            self._call(first, n_steps, ns, _lib.SURV_PRIME_NONE)
             self.surv.peers = None
             self._all_reduce(self.sums[(first + n_steps) & 1])
         else:
             for t in range(first, first + n_steps):
                 if not self._primed:
-                    self._launch(t, 1, ns, _lib.SURV_PRIME_ONLY)
+                    self._call(t, 1, ns, _lib.SURV_PRIME_ONLY)
                     self._all_reduce(self.sums[t & 1])
                     self._primed = True
-                self._launch(t, 1, ns, _lib.SURV_PRIME_NONE)
+                self._call(t, 1, ns, _lib.SURV_PRIME_NONE)
                 if apply_update:
                     self._all_reduce(self.sums[(t + 1) & 1])  # the exchange step: R + 1 doubles per SVI step
         self._primed = True
-        if apply_update:
-            self.step += n_steps
-        return self.loss[first:first + n_steps]
+        return ns[2]
 
-    def gradients(self, noise=None) -> Dict[str, torch.Tensor]:
-        """Loss and its gradient w.r.t. the unconstrained parameters at the current point (no update)."""
-        loss = self.run(1, noise=noise, apply_update=False)
-        return {"loss": loss[0].clone(), "mu_loc": self.var_grad[0].clone(), "mu_scale": self.var_grad[1].clone(),
-                "alpha_pi": self.alpha_grad.clone(), "q0": self.q0_grad.clone()}
+    def _grads(self):
+        return {"mu_loc": self.var_grad[0], "mu_scale": self.var_grad[1], "alpha_pi": self.alpha_grad, "q0": self.q0_grad}
 
     def params(self) -> Dict[str, torch.Tensor]:
         """Constrained parameter values under the reference's names and shapes."""
         T = self.T
         return {"mu_loc": self.var_params[0].reshape(T, 1).clone(), "mu_scale": self.var_params[1].exp().reshape(T, 1),
                 "alpha_pi": self.alpha_u.exp(), "q0": self.q0_u.exp()}
-
-    def losses(self):
-        return self.loss[: self.step].cpu()

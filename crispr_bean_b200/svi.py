@@ -14,13 +14,13 @@ import torch
 
 from . import _lib
 from .device_pack import DeviceScreen, row_constants
-from .halt import NonfiniteWatch
+from .fused import FusedEngine, set_prior_pointers, svi_config
 
 _RUN = {torch.float32: "bean_svi_run_f32", torch.float64: "bean_svi_run_f64"}
 VAR_PARAM_NAMES = ("mu_loc", "mu_scale", "sd_loc", "sd_scale")  # rows of var_params; scales stored as log
 
 
-class SviEngine(NonfiniteWatch):
+class SviEngine(FusedEngine):
     """Parameters + optimiser state + the fused step for one (screen, model) pair on one GPU.
 
     model: "Normal" | "ControlNormal" | "MixtureNormal".  Parameter names, shapes and initial values
@@ -33,12 +33,11 @@ class SviEngine(NonfiniteWatch):
                  seed: int = 101, alpha_prior: float = 1.0, sd_scale: float = 0.01, mask_thres: int = 10,
                  prior_params: Optional[dict] = None, screen: Optional[DeviceScreen] = None,
                  guide_offset: int = 0, variant_offset: int = 0, scale_by_accessibility: bool = False,
-                 fit_noise: bool = False, split: bool = True):
+                 fit_noise: bool = False):
         if model not in ("Normal", "ControlNormal", "MixtureNormal"):
             raise ValueError(f"SviEngine does not implement model {model!r}")
-        self.lib = _lib.lib()
-        self.model, self.dtype, self.device = model, dtype, torch.device(device)
-        self.num_steps = int(num_steps)
+        self._setup(device, dtype, num_steps)
+        self.model = model
         self.mixture = model == "MixtureNormal"
         use_bcmatch = bool(use_bcmatch) and getattr(data, "X_bcmatch_masked", None) is not None
         self.screen = screen or DeviceScreen(data, self.device, dtype=dtype, use_bcmatch=use_bcmatch, mask_thres=mask_thres)
@@ -82,48 +81,14 @@ class SviEngine(NonfiniteWatch):
             self.noise_m, self.noise_v = torch.zeros((2, G), **kw), torch.zeros((2, G), **kw)
             self.noise_grad = torch.zeros((2, G), **kw)
         self.partial = torch.zeros((self.lib.bean_svi_num_partials(G, T),), dtype=torch.float64, device=dev)
-        self.counter = torch.zeros((1,), dtype=torch.int32, device=dev)
-        # one spare slot: `gradients()` evaluates a step without updating and writes its loss at index `step`, which is
-        # num_steps after a complete run
-        self.loss = torch.zeros((max(self.num_steps, 1) + 1,), dtype=torch.float64, device=dev)
-        self.step = 0
 
-        c = _lib.BeanSviConfig()
+        c, self._prior_v = svi_config(lr=initial_lr, gamma=gamma, num_steps=self.num_steps, seed=seed, ll_const=ll_const,
+                                      guide_offset=guide_offset, variant_offset=variant_offset,
+                                      sd_scale=1.0 if model == "ControlNormal" else float(sd_scale), prior_params=prior_params,
+                                      n_variants=T, device=dev, dtype=dtype, pi_a0=getattr(data, "pi_a0", None))
         c.model = _lib.MODEL_MIXTURE_NORMAL if self.mixture else _lib.MODEL_NORMAL
         c.sd_is_sqrt = 1 if model == "Normal" else 0
-        c.apply_update = 1
         c.fit_noise = 1 if self.fit_noise else 0
-        c.mu_prior_normal, c.mu_prior_loc, c.mu_prior_scale = 0, 0.0, 1.0
-        c.sd_prior_loc, c.sd_prior_scale = 0.0, (1.0 if model == "ControlNormal" else float(sd_scale))
-        self._prior_v = {}
-        if prior_params:
-            # scalars or per-variant tensors (T,) / (T, 1), as `bean build-prior` writes them (run.py:480-542)
-            def put(key, field):
-                val = prior_params[key]
-                if torch.is_tensor(val) and val.numel() > 1:
-                    if val.numel() != T:
-                        raise ValueError(f"prior_params[{key!r}] has {val.numel()} entries for {T} variants")
-                    self._prior_v[key] = val.detach().reshape(-1).to(**kw).contiguous()
-                else:
-                    setattr(c, field, float(val))
-
-            if "mu_loc" in prior_params or "mu_scale" in prior_params:
-                c.mu_prior_normal = 1
-                c.mu_prior_loc, c.mu_prior_scale = 0.0, 1.0
-                for key in ("mu_loc", "mu_scale"):
-                    if key in prior_params:
-                        put(key, f"mu_prior_{key[3:]}")
-            for key in ("sd_loc", "sd_scale"):
-                if key in prior_params:
-                    put(key, f"sd_prior_{key[3:]}")
-        c.lr0, c.lrd = float(initial_lr), float(gamma) ** (1.0 / max(self.num_steps, 1))
-        c.beta1, c.beta2, c.adam_eps, c.clip = 0.9, 0.999, 1e-8, 10.0
-        c.ll_const, c.seed = ll_const, int(seed)
-        # Multinomial prob clamp: eps of the dtype pi has in the reference = dtype of pi_a0 (float64 out of the fit)
-        pa0 = getattr(data, "pi_a0", None)
-        ref_dtype = torch.float64 if (dtype == torch.float64 or pa0 is None or not torch.is_tensor(pa0)) else pa0.dtype
-        c.prob_clamp_eps = float(torch.finfo(ref_dtype).eps)
-        c.guide_offset, c.variant_offset = int(guide_offset), int(variant_offset)
         self.cfg = c
 
         s = _lib.BeanSviState()
@@ -136,15 +101,11 @@ class SviEngine(NonfiniteWatch):
         s.var_params, s.var_m, s.var_v = self.var_params.data_ptr(), self.var_m.data_ptr(), self.var_v.data_ptr()
         s.d_guide, s.var_grad = self.d_guide.data_ptr(), self.var_grad.data_ptr()
         s.partial, s.counter, s.loss = self.partial.data_ptr(), self.counter.data_ptr(), self.loss.data_ptr()
-        self.split = bool(split) and self.mixture
-        if self.split:  # scratch of the two-kernel guide step (include/bean_b200.h: pw, dconc)
+        if self.mixture:  # hand-over scratch of the two-kernel guide step (include/bean_b200.h: pw, dconc)
             self.pw = torch.empty((R, G, 4), **kw)
             self.dconc = torch.empty((G, 4), **kw)
             s.pw, s.dconc = self.pw.data_ptr(), self.dconc.data_ptr()
-        for key, field in (("mu_loc", "mu_prior_loc_v"), ("mu_scale", "mu_prior_scale_v"), ("sd_loc", "sd_prior_loc_v"),
-                           ("sd_scale", "sd_prior_scale_v")):
-            if key in self._prior_v:
-                setattr(s, field, self._prior_v[key].data_ptr())
+        set_prior_pointers(s, self._prior_v)
         if self.acc:
             s.acc_k = self.acc_k.data_ptr()
             s.noise_u, s.noise_m, s.noise_v = self.noise_u.data_ptr(), self.noise_m.data_ptr(), self.noise_v.data_ptr()
@@ -153,52 +114,31 @@ class SviEngine(NonfiniteWatch):
         self.state = s
 
     # ---------------------------------------------------------------------------------------------
-    def _noise_struct(self, noise: Optional[Dict[str, torch.Tensor]]):
-        if noise is None:
-            return None, ()
-        kw = dict(device=self.device, dtype=self.dtype)
-        n, keep = _lib.BeanSviNoise(), []
-        if noise.get("record"):  # have the kernels write out the Philox draws they used
-            self.eps_used = torch.zeros((2, self.T), **kw)
-            n.eps_out = self.eps_used.data_ptr()
-            if self.mixture:
-                self.pi_used = torch.zeros((self.screen.n_guides, self.screen.n_reps, 2), **kw)
-                n.pi_out = self.pi_used.data_ptr()
-        if "eps_mu" in noise:
-            em = noise["eps_mu"].reshape(-1).to(**kw).contiguous()
-            es = noise["eps_sd"].reshape(-1).to(**kw).contiguous()
-            assert em.numel() == self.T == es.numel()
-            n.eps_mu, n.eps_sd = em.data_ptr(), es.data_ptr()
-            keep += [em, es]
-        if self.acc and "eps_noise" in noise:
-            en = noise["eps_noise"].reshape(-1).to(**kw).contiguous()
-            assert en.numel() == self.screen.n_guides
-            n.eps_noise = en.data_ptr()
-            keep.append(en)
-        if self.mixture and "pi" in noise:
-            pi = noise["pi"]
-            if pi.dim() == 4:  # reference layout (R, 1, G, 2)
-                pi = pi[:, 0].permute(1, 0, 2)
-            pi = pi.to(**kw).contiguous()
-            assert pi.shape == (self.screen.n_guides, self.screen.n_reps, 2)
-            n.pi = pi.data_ptr()
-            keep.append(pi)
-        return n, keep
-
-    def run(self, n_steps: int, noise: Optional[Dict[str, torch.Tensor]] = None, apply_update: bool = True):
-        """Advance `n_steps` SVI steps (asynchronously); injected `noise` applies to every one of them."""
-        if self.step + n_steps > self.loss.numel() - (1 if apply_update else 0):
-            raise ValueError("loss buffer exhausted: construct the engine with a larger num_steps")
-        n, keep = self._noise_struct(noise)
-        self.cfg.apply_update = 1 if apply_update else 0
+    def _launch(self, first, n_steps, noise, apply_update):
+        n, keep = None, []
+        if noise is not None:
+            n = _lib.BeanSviNoise()
+            if noise.get("record"):  # have the kernels write out the Philox draws they used
+                kw = dict(device=self.device, dtype=self.dtype)
+                self.eps_used = torch.zeros((2, self.T), **kw)
+                n.eps_out = self.eps_used.data_ptr()
+                if self.mixture:
+                    self.pi_used = torch.zeros((self.screen.n_guides, self.screen.n_reps, 2), **kw)
+                    n.pi_out = self.pi_used.data_ptr()
+            if "eps_mu" in noise:
+                self._put(keep, n, "eps_mu", noise["eps_mu"].reshape(-1), (self.T,))
+                self._put(keep, n, "eps_sd", noise["eps_sd"].reshape(-1), (self.T,))
+            if self.acc and "eps_noise" in noise:
+                self._put(keep, n, "eps_noise", noise["eps_noise"].reshape(-1), (self.screen.n_guides,))
+            if self.mixture and "pi" in noise:
+                pi = noise["pi"]
+                if pi.dim() == 4:  # reference layout (R, 1, G, 2)
+                    pi = pi[:, 0].permute(1, 0, 2)
+                self._put(keep, n, "pi", pi, (self.screen.n_guides, self.screen.n_reps, 2))
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        rc = getattr(self.lib, _RUN[self.dtype])(self.screen.c, self.state, self.cfg, n, self.step, n_steps, stream)
+        rc = getattr(self.lib, _RUN[self.dtype])(self.screen.c, self.state, self.cfg, n, first, n_steps, stream)
         _lib.check(rc, _RUN[self.dtype])
-        first = self.step
-        if apply_update:
-            self.step += n_steps
-        self._keep = keep  # keep injected buffers alive until the stream has consumed them
-        return self.loss[first:first + n_steps]
+        return keep
 
     def _snapshot_tensors(self):
         out = [self.var_params, self.var_m, self.var_v]
@@ -208,16 +148,12 @@ class SviEngine(NonfiniteWatch):
             out += [self.noise_u, self.noise_m, self.noise_v]
         return out
 
-    def gradients(self, noise=None) -> Dict[str, torch.Tensor]:
-        """Loss and its gradient w.r.t. the unconstrained parameters at the current point (no update)."""
-        loss = self.run(1, noise=noise, apply_update=False)
-        out = {"loss": loss[0].clone()}
-        for i, k in enumerate(VAR_PARAM_NAMES):
-            out[k] = self.var_grad[i].clone()
+    def _grads(self):
+        out = dict(zip(VAR_PARAM_NAMES, self.var_grad))
         if self.mixture:
-            out["alpha_pi"] = self.alpha_grad.clone()
+            out["alpha_pi"] = self.alpha_grad
         if self.fit_noise:
-            out["noise_loc"], out["noise_scale"] = self.noise_grad[0].clone(), self.noise_grad[1].clone()
+            out["noise_loc"], out["noise_scale"] = self.noise_grad[0], self.noise_grad[1]
         return out
 
     def params(self) -> Dict[str, torch.Tensor]:
@@ -232,6 +168,3 @@ class SviEngine(NonfiniteWatch):
         if self.fit_noise:
             out["noise_loc"], out["noise_scale"] = self.noise_u[0].clone(), self.noise_u[1].exp()
         return out
-
-    def losses(self):
-        return self.loss[: self.step].cpu()

@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define BEAN_ABI_VERSION 16
+#define BEAN_ABI_VERSION 17
 
 enum {
   BEAN_OK = 0,
@@ -158,8 +158,8 @@ int bean_allele_scatter_f64(const BeanAlleleMap* map, const void* sd_edit, const
  *   Trace_ELBO (1 particle) loss and its gradient (pyro.infer; pathwise Dirichlet derivative as
  *       torch._dirichlet_grad), then pyro.optim.ClippedAdam on the unconstrained parameters.
  * Kernels per step: a per-guide kernel (sampling, likelihood, editing-rate sites, per-guide d/d(mu, sd)), for the mixture
- * model a second per-guide kernel (pathwise Dirichlet derivative of every draw, alpha_pi gradient and its Adam update;
- * folded into the first when BeanSviState.pw / dconc are NULL) and a per-variant kernel (segmented reduction of the
+ * model a second per-guide kernel (pathwise Dirichlet derivative of every draw, alpha_pi gradient and its Adam update,
+ * from what the first leaves in BeanSviState.pw / dconc) and a per-variant kernel (segmented reduction of the
  * guide gradients over the CSR variant ranges, prior / entropy terms, Adam on the variant parameters, loss).
  *
  * Randomness is counter-based (Philox4x32-10 keyed by `seed`, indexed by (entity, replicate, step)),
@@ -175,7 +175,7 @@ typedef struct BeanSviConfig {
   int32_t mu_prior_normal;  /* 0: Laplace(0,1) (model.py:43); 1: Normal(mu_prior_loc, mu_prior_scale) */
   int32_t apply_update;     /* 1: ClippedAdam step; 0: only write gradients                          */
   int32_t phases;           /* 0: the whole step; otherwise a bit mask -- 1 guide kernel, 2 variant kernel, 4 alpha kernel
-                               (split guide step only) -- so a benchmark can time each kernel with CUDA events */
+                               (MIXTURE only) -- so a benchmark can time each kernel with CUDA events */
   int32_t fit_noise;        /* --scale-by-acc only: 1 = guide Normal(noise_loc, noise_scale) on logit_pi_noise
                                (utils.py:145-155), 0 = drawn from the prior Normal(0, 0.655)           */
   int32_t force_generic;    /* 1: never pick the specialised kernels (exactly 4 / 5 bins, no masked sample); tests use it
@@ -225,8 +225,8 @@ typedef struct BeanSviState {
   const void* mu_prior_scale_v;  /* real [T] */
   const void* sd_prior_loc_v;    /* real [T] */
   const void* sd_prior_scale_v;  /* real [T] */
-  /* optional scratch of the split guide step (MIXTURE): when both are non-NULL the pathwise Dirichlet derivative and
-     the alpha_pi update run in a second kernel that reads what the first one leaves here                          */
+  /* scratch of the MIXTURE guide step, required there (BEAN_EINVAL when NULL), 16-byte aligned: the first per-guide kernel
+     leaves here what the second one (pathwise Dirichlet derivative, alpha_pi update) reads                           */
   void* pw;                      /* real [R][G][4]: (pi0, pi1, w0, w1) of every draw (replicate-major: coalesced)    */
   void* dconc;                   /* real [G][4]:    concentration gradients without the pathwise part               */
   /* device i32 [1] or NULL (off): first non-finite step.  A step t that runs with apply_update = 1 and whose loss[t] or any

@@ -16,7 +16,7 @@ from crispr_bean_b200.svi import SviEngine
 data = build_data("c5_genome_scale", 101)
 dev = torch.device("cuda")
 N = int(sys.argv[1]) if len(sys.argv) > 1 else 2000
-eng = SviEngine(data, "MixtureNormal", dev, num_steps=N, split=os.environ.get("BEAN_SPLIT", "1") == "1")
+eng = SviEngine(data, "MixtureNormal", dev, num_steps=N)
 for blk in range(N // 100):
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     a.record(); eng.run(100); b.record(); torch.cuda.synchronize()

@@ -277,23 +277,6 @@ def test_end_to_end_result_table_equals_oracle_run(cuda_device):
         assert (tab_gpu[c] - tab_ref[c]).abs().max() <= 1e-7 * tab_ref[c].abs().max(), c
 
 
-@pytest.mark.parametrize("dtype,rtol", [(torch.float64, 1e-11), (torch.float32, 2e-4)])
-def test_split_and_fused_guide_step_agree(cuda_device, dtype, rtol):
-    """The two-kernel guide step (svi_guide_kernel + svi_alpha_kernel, default) and the single-kernel one (no hand-over
-    scratch) are the same computation: same Philox draws, same loss, same parameters after a few steps (the pathwise terms
-    are only summed in a different order)."""
-    data = H.make_small_mixture_data(n_variants=50, n_reps=4, seed=17)
-    runs = []
-    for split in (True, False):
-        eng = SviEngine(data, "MixtureNormal", cuda_device, dtype=dtype, num_steps=10, seed=3, split=split)
-        assert eng.split == split
-        eng.run(6)
-        runs.append((eng.losses(), {k: v.cpu() for k, v in eng.params().items()}))
-    torch.testing.assert_close(runs[0][0], runs[1][0], rtol=1e-9 if dtype == torch.float64 else 1e-6, atol=0)
-    for k, v in runs[0][1].items():
-        torch.testing.assert_close(v, runs[1][1][k], rtol=rtol, atol=rtol * 1e-2)
-
-
 def test_sampler_distribution_probability_integral_transform(cuda_device):
     """Every recorded pi draw pushed through ITS OWN Beta CDF must be uniform (Kolmogorov-Smirnov), across concentrations
     from 1e-2 (Marsaglia-Tsang boost path, draws piling up at the clamps) to 1e3; and the Normal draws must be normal."""

@@ -1,5 +1,5 @@
-"""Where the fp32 alpha_pi error of the reference's var_mini screen comes from: the fused step with the guide kernel split / not
-split / unspecialised, worst elements with their concentrations and draws.  GPU diagnostic; prints JSON lines."""
+"""Where the fp32 alpha_pi error of the reference's var_mini screen comes from: the fused step in float32 and
+float64, worst elements with their concentrations and draws.  GPU diagnostic; prints JSON lines."""
 import json
 import os
 import sys
@@ -20,9 +20,8 @@ perm = edit_perm(z, data)
 noise = {k: torch.as_tensor(to_ours(v, perm, k)) for k, v in group(z, "native/noise/").items() if "/" not in k}
 ref = np.asarray(truth["grads"]["alpha_pi"]).reshape(-1, 2)
 scale = np.maximum(np.abs(ref), 1e-3 * np.abs(ref).max())
-for label, kw, dtype in (("split", dict(split=True), torch.float32), ("nosplit", dict(split=False), torch.float32),
-                         ("f64", dict(split=True), torch.float64)):
-    eng = SviEngine(data, "MixtureNormal", dev, dtype=dtype, num_steps=4, **kw)
+for label, dtype in (("f32", torch.float32), ("f64", torch.float64)):
+    eng = SviEngine(data, "MixtureNormal", dev, dtype=dtype, num_steps=4)
     got = eng.gradients(noise)["alpha_pi"].detach().double().cpu().numpy().reshape(-1, 2)
     err = np.abs(got - ref) / scale
     order = np.argsort(-err.max(1))[:4]

@@ -21,19 +21,17 @@ def main():
     ap.add_argument("--burn-in", type=int, default=300)
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--tag", default="")
-    ap.add_argument("--no-split", action="store_true", help="single-kernel guide step (no hand-over to svi_alpha_kernel)")
     args = ap.parse_args()
     dev = torch.device("cuda:0")
     data = build_data(args.workload, seed=101)
-    eng = SviEngine(data, "MixtureNormal", dev, dtype=torch.float32, num_steps=args.burn_in + 20 * args.steps + 64, seed=101,
-                    split=not args.no_split)
+    eng = SviEngine(data, "MixtureNormal", dev, dtype=torch.float32, num_steps=args.burn_in + 20 * args.steps + 64, seed=101)
     out = {"tag": args.tag, "workload": args.workload, "guides": data.n_guides}
     for label, burn in (("early", 5), ("steady", args.burn_in)):
         eng.run(max(burn - eng.step, 0))
         eng.run(3)
         full = time_steps(eng, args.steps) / args.steps
         g = time_steps(eng, args.steps, phases=1) / args.steps
-        a = time_steps(eng, args.steps, phases=4) / args.steps if eng.split else 0.0
+        a = time_steps(eng, args.steps, phases=4) / args.steps
         v = time_steps(eng, args.steps, phases=2) / args.steps
         out[label] = {"step_ms": round(full, 4), "guide_ms": round(g, 4), "alpha_ms": round(a, 4), "variant_ms": round(v, 4)}
     out["loss"] = float(eng.loss[eng.step - 1])
