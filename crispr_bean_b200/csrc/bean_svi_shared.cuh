@@ -201,17 +201,17 @@ __device__ __forceinline__ void grid_dependency_wait() {
 #endif
 }
 template <typename Kernel, typename Params>
-static inline void launch_after(Kernel kernel, int grid, int block, cudaStream_t st, const Params& p) {
+static inline void launch_after(Kernel kernel, int grid, int block, cudaStream_t st, const Params& p, size_t smem = 0) {
 #ifdef BEAN_PDL
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)block); cfg.dynamicSmemBytes = 0; cfg.stream = st;
+  cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)block); cfg.dynamicSmemBytes = smem; cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
   cudaLaunchKernelEx(&cfg, kernel, p);
 #else
-  kernel<<<grid, block, 0, st>>>(p);
+  kernel<<<grid, block, smem, st>>>(p);
 #endif
 }
 

@@ -89,9 +89,10 @@ def _halt(eng, snap, t: int, batch_start: int, collect: Callable, rank: int):
 
 
 def make_engine(model, guide, data, initial_lr=0.01, gamma=0.1, num_steps=2000, device="cuda", dtype=torch.float32,
-                seed=101, guide_offset=0, variant_offset=0):
+                seed=101, guide_offset=0, variant_offset=0, replica=False):
     """The device-resident SVI engine of a (model, guide) pair.  `guide_offset` / `variant_offset`: global index of the first
-    guide / variant of `data` when it is one shard of a larger screen (the noise counters use global ids)."""
+    guide / variant of `data` when it is one shard of a larger screen (the noise counters use global ids).  `replica`: `data` is
+    the whole screen, fitted by this process alone even when torch.distributed has more than one rank (no collectives)."""
     name, mkw = resolve(model)
     gname, gkw = resolve(guide)
     if name != gname:
@@ -127,9 +128,10 @@ def make_engine(model, guide, data, initial_lr=0.01, gamma=0.1, num_steps=2000, 
         from .generic import TilingSviEngine
         from . import tiling_fused
 
-        if tiling_fused.supports(data, scale_by_acc):  # <= 32 alleles per guide, no --scale-by-acc
+        # 2..1024 alleles per guide, no --scale-by-acc, and (above 32 alleles) small enough for the fused step to be faster
+        if tiling_fused.serves(data, scale_by_acc) and tiling_fused.faster_than_site_kernels(data):
             return tiling_fused.TilingFusedEngine(data, use_bcmatch=True, alpha_prior=alpha_prior, sd_scale=sd_scale, epsilon=epsilon,
-                                                  guide_offset=guide_offset, **kw)
+                                                  guide_offset=guide_offset, sharded=False if replica else None, **kw)
         return TilingSviEngine(data, use_bcmatch=True, alpha_prior=alpha_prior, sd_scale=sd_scale, epsilon=epsilon,
                                scale_by_accessibility=scale_by_acc, fit_noise=fit_noise, **kw)
     if name == "Normal" and getattr(data, "sample_covariates", None) is not None:
@@ -184,7 +186,8 @@ def run_inference(model, guide, data, initial_lr=0.01, gamma=0.1, num_steps=2000
 
         params, loss = run_sharded(make, data, num_steps, tdist.get_rank(), world, log_every=log_every)
         return params, {"loss": loss.tolist(), "params": {k: v.detach().cpu() for k, v in params.items()}}
-    eng = make_engine(model, guide, data, initial_lr, gamma, num_steps, device, dtype, seed)
+    # every rank fits the whole screen (a replica): its engine must not all-reduce with the other ranks
+    eng = make_engine(model, guide, data, initial_lr, gamma, num_steps, device, dtype, seed, replica=True)
     params, losses = run_batches(eng, num_steps, log_every)
     return params, {"loss": losses.tolist(), "params": {k: v.detach().cpu() for k, v in params.items()}}
 

@@ -1,12 +1,16 @@
 """Device-resident SVI engine of the tiling sorting program (MultiMixtureNormal): host side of `bean_svi_tiling_run_*`.
 
 One step = `svi.step` of bean/model/run.py:376-380 for bean/model/model.py:550-751 / :878-962 in three kernel launches
-(per-edit draws, warp-per-guide kernel with a lane per allele, per-edit reduction + update; include/bean_b200.h), no torch
-op and no host round trip per step.  Parameter names, shapes and initial values follow the pyro guide (model.py:893-937):
+(per-edit draws, CTA-per-guide kernel, per-edit reduction + update; include/bean_b200.h), no torch op and no host round trip
+per step.  Parameter names, shapes and initial values follow the pyro guide (model.py:893-937):
 mu_loc = 0, mu_scale = 1, sd_loc = 0, sd_scale = 1 (E,), alpha_pi = alpha_prior (G, A) with epsilon at non-existent alleles.
 
-Takes designs with at most 32 alleles per guide (one lane per allele: filtered allele tables; wider raw tables and
-`--scale-by-acc` stay on `generic.TilingSviEngine`) -- see `supports()`.
+Takes designs with 2..1024 alleles per guide (`serves()`): up to 32 (filtered allele tables) the guide kernel gives each
+allele a lane, from 33 on (raw tables, e.g. 231 in the reference's tiling_mini screen) each lane walks alleles l, l + 32, ...
+with the per-allele values in shared memory.  `--scale-by-acc` and wider tables stay on `generic.TilingSviEngine`, and so do
+wide designs with more allele draws per step than the fused step is measured faster for (`faster_than_site_kernels`).
+`supports()` is the narrower set the guide blocks of a screen are sharded over ranks for (`run.shards_over_ranks`): at most
+32 alleles.  Wider screens run as replicas, unsharded on every rank.
 """
 from __future__ import annotations
 
@@ -21,25 +25,48 @@ from .fused import FusedEngine, dist_active, pi_dtype, set_prior_pointers, svi_c
 from .tiling import AlleleMap
 
 _RUN = {torch.float32: "bean_svi_tiling_run_f32", torch.float64: "bean_svi_tiling_run_f64"}
-MAX_ALLELES = 32
+MAX_ALLELES = 32  # one lane per allele; the widest design sharded over ranks
+MAX_WIDE_ALLELES = 1024  # BEAN_TILING_FUSED_MAX_ALLELES
 
 
 def supports(data, scale_by_accessibility: bool = False) -> bool:
+    """At most 32 alleles per guide, no --scale-by-acc: the designs whose guide blocks shard over ranks."""
     return (not scale_by_accessibility) and 2 <= int(data.n_max_alleles) <= MAX_ALLELES
+
+
+def serves(data, scale_by_accessibility: bool = False) -> bool:
+    """Whether the fused step runs this design: 2..1024 alleles per guide, no --scale-by-acc."""
+    return (not scale_by_accessibility) and 2 <= int(data.n_max_alleles) <= MAX_WIDE_ALLELES
+
+
+# Above 32 alleles the guide kernel is bound by the latency of each guide's chain of R x A double-precision draws, with fewer
+# guides resident per SM as A grows (shared memory), while the site-kernel engine spreads the draws over all threads.  On a
+# B200 the fused step is the faster of the two up to about this many allele draws per step (n_guides x n_reps x n_alleles;
+# profiles/tiling_wide_timings.json), and `run.make_engine` sends wider work to the site-kernel engine.
+WIDE_MAX_DRAWS = 400_000
+
+
+def faster_than_site_kernels(data) -> bool:
+    """Whether the fused step is measured faster than `generic.TilingSviEngine` for a design it serves."""
+    A = int(data.n_max_alleles)
+    return A <= MAX_ALLELES or int(data.n_guides) * int(data.n_reps) * A <= WIDE_MAX_DRAWS
 
 
 class TilingFusedEngine(FusedEngine):
     def __init__(self, data, device="cuda", dtype=torch.float32, use_bcmatch: bool = True, num_steps: int = 2000,
                  initial_lr: float = 0.01, gamma: float = 0.1, seed: int = 101, alpha_prior: float = 1.0, sd_scale: float = 0.01,
-                 epsilon: float = 1e-5, prior_params: Optional[dict] = None, guide_offset: int = 0, group=None):
+                 epsilon: float = 1e-5, prior_params: Optional[dict] = None, guide_offset: int = 0, group=None,
+                 sharded: Optional[bool] = None):
         if not torch.cuda.is_available():
             raise _lib.BeanError("TilingFusedEngine needs a CUDA device: there is no CPU fallback")
-        if not supports(data):
-            raise ValueError(f"the fused tiling step takes 2..{MAX_ALLELES} alleles per guide (got {data.n_max_alleles})")
+        if not serves(data):
+            raise ValueError(f"the fused tiling step takes 2..{MAX_WIDE_ALLELES} alleles per guide (got {data.n_max_alleles})")
         self._setup(device, dtype, num_steps)
         self.model = "MultiMixtureNormal"
-        # guides sharded over the ranks of `group` (dist.shard_data): `data` is this rank's guide block with ALL edits of the screen
-        self.group, self.sharded = group, dist_active(group)
+        # guides sharded over the ranks of `group` (dist.shard_data): `data` is this rank's guide block with ALL edits of the screen.
+        # sharded=None: whenever `group` has more than one rank; sharded=False: a replica fitting the whole screen on its own
+        self.group = group
+        self.sharded = dist_active(group) if sharded is None else (bool(sharded) and dist_active(group))
         self.replicated_params = ("mu_loc", "mu_scale", "sd_loc", "sd_scale")  # per edit: identical on every rank
         use_bcmatch = bool(use_bcmatch) and getattr(data, "X_bcmatch_masked", None) is not None
         self.screen = DeviceScreen(data, self.device, dtype=dtype, use_bcmatch=use_bcmatch, mask_thres=10)

@@ -47,6 +47,7 @@ enum { BEAN_MODE_SORTING = 0, BEAN_MODE_SURVIVAL = 1 };
 #define BEAN_MAX_BINS 8        /* n_condits incl. the control pseudo-bin (SURVEY App. B1) */
 #define BEAN_MAX_RB 64         /* n_reps * n_bins per guide */
 #define BEAN_MAX_ALLELES 4096  /* alleles per guide incl. wild type (raw tiling allele tables reach hundreds) */
+#define BEAN_TILING_FUSED_MAX_ALLELES 1024 /* alleles per guide incl. wild type in bean_svi_tiling_run_* */
 #define BEAN_MAX_LAYERS 2
 #define BEAN_SURV_FOLD_ROWS 1024 /* spare rows of BeanSurvivalState.abund_partial (second level of the abundance sums) */
 #define BEAN_MAX_PEERS 8        /* GPUs of one box */
@@ -343,8 +344,9 @@ int bean_row_const_f64(const void* x, int64_t n_rows, int32_t n_bins, int32_t wi
  * non-existent alleles forced to 0; `pi` ~ Dirichlet over the alleles of a guide; allele mixture; get_alpha +
  * Dirichlet-Multinomial sites; `pi` Dirichlet prior with the epsilon-regularised concentration, guide Dirichlet and
  * `bulk_allele_count` Multinomial under repguide_mask; Trace_ELBO loss and gradient; ClippedAdam.  Three launches per step:
- * per-edit draws, a warp-per-guide kernel with one lane per allele (so n_alleles <= 32: filtered allele tables; wider raw
- * tables stay on the site-kernel engine), and the per-edit kernel that reduces the allele slots over the CSC map.
+ * per-edit draws, a CTA-per-guide kernel, and the per-edit kernel that reduces the allele slots over the CSC map.  The guide
+ * kernel gives each allele a lane for n_alleles <= 32 (filtered allele tables); for 33..BEAN_TILING_FUSED_MAX_ALLELES (raw
+ * tables) lane l walks the alleles l, l + 32, ... with the per-allele values in shared memory.  Other widths: BEAN_EINVAL.
  * Without --scale-by-acc.  Layouts: alpha_u / alpha_m / alpha_v / allele_mask [G][A]; counts [R][C][G][A]; pi [R][G][A].
  * ---------------------------------------------------------------------------------------------- */
 typedef struct BeanTilingState {
